@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PPO hot path (BASELINE.json metric: env-steps/sec, PPO update included).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--epochs E] [--engine auto|simt|tcgen05]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--epochs E] [--engine auto|simt|tcgen05] [--dump-outputs DIR]
 
 One "step" = one full PPO iteration of BASELINE config 2 per GPU: 128 rollout steps of 4096 synthetic Box(376)/Box(17)
 envs (policy+critic forward, sampling, buffer writes), bootstrap values + GAE, then nr_epochs x (B / minibatch) shuffled
@@ -149,6 +149,24 @@ def timed_iterations(model, steps, dist):
     if dist is not None:
         dist.barrier()
     return e0.elapsed_time(e1) / 1e3, t0, t1
+
+
+DUMP_ENV_SAMPLE = 512   # env columns kept of the [T, N, act_dim] actions (seeded choice), so that the whole dump stays far below 64 MB
+
+
+def dump_outputs(model, out_dir):
+    """What the last timed iteration handed to a caller, as float32 .npy files: the updated parameters and Adam moments, the per-minibatch
+    metric records, and the rollout buffer (per-(step, env) arrays in full, actions for a fixed seeded sample of env columns)."""
+    os.makedirs(out_dir, exist_ok=True)
+    torch.cuda.synchronize()
+    b = model.batch
+    cols = np.sort(np.random.default_rng(0).choice(b.actions.shape[1], size=min(DUMP_ENV_SAMPLE, b.actions.shape[1]), replace=False))
+    arrays = {"params": model.params.flat, "adam_exp_avg": model.exp_avg, "adam_exp_avg_sq": model.exp_avg_sq, "metrics": model.metrics_dev,
+              "log_probs": b.log_probs, "values": b.values, "rewards": b.rewards, "terminations": b.terminations, "advantages": b.advantages,
+              "returns": b.returns, "actions_env_sample": b.actions[:, torch.from_numpy(cols).to(b.actions.device)], "actions_env_sample_index": cols}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else t
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def available_cores():
@@ -679,6 +697,8 @@ def main():
     ap.add_argument("--no-parity-check", action="store_true", help="N>1: skip the sharded-vs-single parity run before timing")
     ap.add_argument("--no-strict", action="store_true", help="N>1: skip the second timed region at the contract's GLOBAL minibatch of 32768")
     ap.add_argument("--global-minibatch", type=int, default=0, help="N>1: headline region with this GLOBAL minibatch instead of --minibatch per GPU")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="PPO workload: write what the last timed step computed to DIR/<name>.npy (rank 0), for output-by-output comparison of two builds")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
@@ -736,6 +756,8 @@ def main():
     seconds, t0, t1 = timed_iterations(model, args.steps, dist)
     launches = int(lib.rlx_launch_count())
     clocks = sampler.stop(t0, t1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(model, args.dump_outputs)
     if dist is not None:
         tt = torch.tensor([seconds], device="cuda")
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)

@@ -3,6 +3,7 @@ import sys
 
 import numpy as np
 import pytest
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
@@ -134,3 +135,78 @@ def emu_build_cmd(out, src):
     import shlex
     return (["g++", "-x", "c++", "-std=c++17", "-O1", "-fPIC", "-shared", "-pthread", "-DRLX_EMU"] + shlex.split(os.environ.get("RLX_EMU_CXXFLAGS", ""))
             + ["-o", str(out), str(src)])
+
+
+def reference_interfaces():
+    """tests/golden/reference_interfaces.json, captured from the executed reference (tests/golden/make_golden_reference_interfaces.py)."""
+    import json
+    with open(os.path.join(GOLDEN_DIR, "reference_interfaces.json")) as fh:
+        return json.load(fh)
+
+
+class _Node(torch.nn.Module):
+    pass
+
+
+def reference_module(layout):
+    """A module with the reference module's parameters and buffers: same names (torch.compile's "_orig_mod." prefix removed), shapes, dtypes
+    and named_parameters() order, so that strict load_state_dict accepts exactly what the reference module accepts."""
+    root = _Node()
+    params = {n for n, _ in layout["parameters"]}
+    for name, shape, dtype in layout["state_dict"]:
+        *path, leaf = name.split(".")
+        node = root
+        for part in path:
+            if not hasattr(node, part):
+                node.add_module(part, _Node())
+            node = getattr(node, part)
+        if name in params:
+            node.register_parameter(leaf, torch.nn.Parameter(torch.zeros(shape, dtype=getattr(torch, dtype))))
+        else:
+            node.register_buffer(leaf, torch.zeros(shape, dtype=getattr(torch, dtype)))
+    assert [[n, list(p.shape)] for n, p in root.named_parameters()] == layout["parameters"]
+    assert [[n, list(t.shape), str(t.dtype).replace("torch.", "")] for n, t in root.state_dict().items()] == layout["state_dict"]
+    return root
+
+
+def reference_optimizer(layout, modules):
+    """The reference's optimizer over the stand-in modules: same class, same param_group settings, parameters in the reference's numbering.
+    `modules`: prefix -> module, the prefixes the captured parameter names carry ("" for an optimizer over one module)."""
+    named = {(f"{prefix}.{n}" if prefix else n): p for prefix, m in modules.items() for n, p in m.named_parameters()}
+    groups = [dict(g["settings"], params=[named[n] for n in g["param_names"]]) for g in layout["param_groups"]]
+    for g in groups:
+        g["betas"] = tuple(g["betas"])
+    return getattr(torch.optim, layout["class"])(groups)
+
+
+def reference_optimizers(ref, mods, ent):
+    """The three optimizers of the reference's SAC / FastSAC over stand-in modules (policy; q1 then q2; the entropy module's log_alpha)."""
+    return {"policy_optimizer": reference_optimizer(ref["optimizers"]["policy_optimizer"], {"": mods["policy"]}),
+            "q_optimizer": reference_optimizer(ref["optimizers"]["q_optimizer"], {"q1": mods["q1"], "q2": mods["q2"]}),
+            "entropy_optimizer": reference_optimizer(ref["optimizers"]["entropy_optimizer"], {"": ent})}
+
+
+def load_like_the_reference(path, ref):
+    """What the reference's SAC / FastSAC load() does with a checkpoint file (sac.py:400-416, fastsac.py:483-500), on stand-in modules and
+    optimizers laid out as the reference's (`ref`: one entry of reference_interfaces.json "checkpoints").  Returns the modules, the
+    optimizers and the entropy module whose log_alpha the file replaced."""
+    ck = torch.load(path, weights_only=False)
+    assert hasattr(ck["config_algorithm"], "items")
+    mods = {name: reference_module(layout) for name, layout in ref["modules"].items()}
+    ent = _Node()
+    ent.log_alpha = torch.nn.Parameter(torch.zeros(ref["log_alpha"]["shape"]))
+    opts = reference_optimizers(ref, mods, ent)
+    for name, mod in mods.items():
+        mod.load_state_dict(ck[f"{name}_state_dict"])
+    ent.log_alpha = ck["log_alpha"]          # a registered parameter: torch accepts only an nn.Parameter here
+    for name, opt in opts.items():
+        opt.load_state_dict(ck[f"{name}_state_dict"])
+    assert set(ck) == set(ref["keys"]) and type(ck["log_alpha"]).__name__ == ref["keys"]["log_alpha"]
+    return mods, opts, ent
+
+
+def reference_enums():
+    """The reference's enum classes as foreign classes: same class names, member names and values (captured from the reference in
+    tests/golden/reference_interfaces.json), defined outside this package."""
+    from enum import Enum
+    return {name: Enum(name, members) for name, members in reference_interfaces()["enums"].items()}

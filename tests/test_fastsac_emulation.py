@@ -381,26 +381,20 @@ def test_plugin_checkpoint_has_the_reference_layout(tmp_path):
 
 
 def test_checkpoints_move_between_the_plugin_and_the_reference_classes(tmp_path):
-    """f2 for FastSAC with the reference's OWN classes (staged copy oracle/_ref, rl_x/algorithms/fastsac/pytorch): (1) a `latest.model`
-    written by the reference's FastSAC.save() (fastsac.py:463-478) after AdamW steps on every parameter is read by the plugin's load() and
-    every tensor - parameters, targets, both AdamW moments, step counts, log_alpha, normaliser statistics - lands on the segment its name
-    says; (2) the file the plugin's save() writes goes through the reference's FastSAC.load() (strict load_state_dict + optimizer
+    """f2 for FastSAC against the reference's checkpoint layout (tests/golden/reference_interfaces.json, captured from the executed
+    reference's FastSAC: file keys, module keys / shapes / dtypes, AdamW numbering and settings): (1) a `latest.model` laid out as the
+    reference's FastSAC.save() writes it (fastsac.py:463-478), after AdamW steps on every parameter, is read by the plugin's load() and every
+    tensor - parameters, targets, both AdamW moments, step counts, log_alpha, normaliser statistics - lands on the segment its name says;
+    (2) the file the plugin's save() writes goes through the reference's load() sequence (strict load_state_dict + optimizer
     load_state_dict, :481-500) and arrives tensor for tensor.  The plugin runs on CPU with the source rewrites of the tests above."""
     import types
-    from oracle import make_ref
-    if not make_ref.available() or not os.path.exists(os.path.join(make_ref.DST, "rl_x", "algorithms", "fastsac", "pytorch", "fastsac.py")):
-        pytest.skip("oracle/_ref (with the FastSAC modules) not staged: python oracle/make_ref.py")
-    from oracle import ref_arm
-    os.environ["TORCHDYNAMO_DISABLE"] = "1"
-    ref_arm.import_reference()
-    import rl_x.algorithms.fastsac.pytorch.fastsac as reffs
-    from rl_x.algorithms.fastsac.pytorch.default_config import get_config as ref_config
-    from rl_x.environments.action_space_type import ActionSpaceType as RA
-    from rl_x.environments.data_interface_type import DataInterfaceType as RD
-    from rl_x.environments.observation_space_type import ObservationSpaceType as RO
+    from conftest import load_like_the_reference, reference_interfaces, reference_module, reference_optimizers
     from rl_x_b200.config_dict import ConfigDict
     from rl_x_b200.algorithms.fastsac.b200.default_config import get_config
-    obs, act, atoms, N = 9, 4, 21, 4
+    from rl_x_b200.environments.types import ActionSpaceType, ObservationSpaceType, DataInterfaceType
+    interfaces = reference_interfaces()
+    layout = interfaces["checkpoints"]["fastsac"]
+    obs, act, atoms, N = (layout["meta"][k] for k in ("obs", "act", "nr_atoms", "nr_envs"))
 
     class Sp:
         def __init__(self, shape, **kw):
@@ -408,7 +402,7 @@ def test_checkpoints_move_between_the_plugin_and_the_reference_classes(tmp_path)
             self.__dict__.update(kw)
 
     class Props:
-        observation_space_type, action_space_type, data_interface_type = RO.FLAT_VALUES, RA.CONTINUOUS, RD.TORCH
+        observation_space_type, action_space_type, data_interface_type = ObservationSpaceType.FLAT_VALUES, ActionSpaceType.CONTINUOUS, DataInterfaceType.TORCH
 
     class Env:
         general_properties, horizon = Props, 3
@@ -416,29 +410,37 @@ def test_checkpoints_move_between_the_plugin_and_the_reference_classes(tmp_path)
         single_action_space = Sp((act,), low=np.full(act, -1.0, np.float32), high=np.full(act, 1.0, np.float32), center=np.zeros(act, np.float32),
                                  scale=np.ones(act, np.float32))
 
-    # ---- the reference model, with optimiser state on every parameter
-    ra = ref_config("fastsac.pytorch")
-    ra.device, ra.bf16_mixed_precision_training, ra.compile_mode, ra.nr_atoms = "cpu", False, "default", atoms
-    rcfg = ref_arm._ConfigDict(algorithm=ra, environment=ref_arm._ConfigDict(seed=8, nr_envs=N),
-                               runner=ref_arm._ConfigDict(save_model=True, track_console=False, track_tb=False, track_wandb=False))
-    ref_run = tmp_path / "ref_run"
-    ref = reffs.FastSAC(rcfg, Env(), Env(), str(ref_run), None)
+    # ---- a file laid out as the reference's save() writes it, with optimiser state on every parameter
     g = torch.Generator().manual_seed(0)
-    for opt in (ref.policy_optimizer, ref.q_optimizer, ref.entropy_optimizer):
+    ref = {name: reference_module(m) for name, m in layout["modules"].items()}
+    ent = torch.nn.Module()
+    ent.log_alpha = torch.nn.Parameter(torch.full(layout["log_alpha"]["shape"], -0.3))
+    with torch.no_grad():
+        for name, m in ref.items():
+            for p in m.parameters():
+                p.copy_(torch.randn(p.shape, generator=g) * 0.1)
+    opts = reference_optimizers(layout, ref, ent)
+    for opt in opts.values():
         for _ in range(3):
             for group in opt.param_groups:
                 for p in group["params"]:
                     p.grad = torch.randn(p.shape, generator=g) * 0.1
             opt.step()
     with torch.no_grad():
-        for tgt in (ref.critic.q1_target, ref.critic.q2_target):
-            for p in tgt.parameters():
-                p.add_(torch.randn(p.shape, generator=g) * 0.01)
-    ref.observation_normalizer.train()
-    ref.observation_normalizer.normalize(torch.randn(32, obs, generator=g) * 2 + 1, update=True)   # non-trivial running statistics
-    os.makedirs(os.path.join(str(ref_run), "models"), exist_ok=True)
-    ref.save()
-    ref_file = os.path.join(str(ref_run), "models", "latest.model")
+        for tgt, src in (("q1_target", "q1"), ("q2_target", "q2")):
+            for p, q in zip(ref[tgt].parameters(), ref[src].parameters()):
+                p.copy_(q + torch.randn(p.shape, generator=g) * 0.01)
+        nrm = ref["observation_normalizer"]
+        nrm.running_mean.copy_(torch.randn(nrm.running_mean.shape, generator=g))                       # non-trivial running statistics
+        nrm.running_var.copy_(torch.rand(nrm.running_var.shape, generator=g) + 0.5)
+        nrm.running_std_dev.copy_(nrm.running_var.sqrt())
+        nrm.count.fill_(32)
+    ra = ConfigDict(dict(interfaces["default_configs"]["fastsac"]))
+    ra.name, ra.device, ra.bf16_mixed_precision_training, ra.compile_mode, ra.nr_atoms = "fastsac.pytorch", "cpu", False, "default", atoms
+    ref_file = str(tmp_path / "latest.model")
+    torch.save({"config_algorithm": ra, **{f"{name}_state_dict": m.state_dict() for name, m in ref.items()}, "log_alpha": ent.log_alpha,
+                **{f"{name}_state_dict": opt.state_dict() for name, opt in opts.items()}}, ref_file)
+    assert set(torch.load(ref_file, weights_only=False)) == set(layout["keys"])
 
     # ---- the plugin class on CPU (device hooks rewritten; only host functions of the library are used)
     src = open(os.path.join(ROOT, "rl_x_b200", "algorithms", "fastsac", "b200", "fastsac.py")).read()
@@ -455,43 +457,37 @@ def test_checkpoints_move_between_the_plugin_and_the_reference_classes(tmp_path)
     ours = mod.FastSAC.load(cfg, Env(), Env(), str(tmp_path / "our_run"), None, [])
     assert int(ours.dims.nr_atoms) == atoms     # taken from the file's config_algorithm
     nq = ours.q_offsets[-1]
-    strip = lambda name: name.replace("_orig_mod.", "")
 
     def check(module, opt, flat, m, v, net, step_index):
         named, nm, nv = ours._named(flat, net), ours._named(m, net) if m is not None else None, ours._named(v, net) if v is not None else None
         for name, p in module.named_parameters():
-            name = strip(name)
             assert torch.equal(named[name], p.detach()), (net, name)
             if opt is not None:
                 st = opt.state[p]
                 assert torch.equal(nm[name], st["exp_avg"]) and torch.equal(nv[name], st["exp_avg_sq"]), (net, name)
                 assert int(ours.steps[step_index]) == int(float(st["step"])) == 3
 
-    check(ref.policy, ref.policy_optimizer, ours.policy_params, ours.policy_m, ours.policy_v, "policy", 2)
-    check(ref.critic.q1, ref.q_optimizer, ours.q_params[:nq], ours.q_m[:nq], ours.q_v[:nq], "q", 0)
-    check(ref.critic.q2, ref.q_optimizer, ours.q_params[nq:], ours.q_m[nq:], ours.q_v[nq:], "q", 0)
-    check(ref.critic.q1_target, None, ours.q_target_params[:nq], None, None, "q", 0)
-    check(ref.critic.q2_target, None, ours.q_target_params[nq:], None, None, "q", 0)
-    la = ref.entropy_coefficient.log_alpha
-    assert torch.equal(ours.log_alpha.reshape(-1), la.detach().reshape(-1))
-    st = ref.entropy_optimizer.state[la]
+    def check_all(ref, opts):
+        check(ref["policy"], opts["policy_optimizer"], ours.policy_params, ours.policy_m, ours.policy_v, "policy", 2)
+        check(ref["q1"], opts["q_optimizer"], ours.q_params[:nq], ours.q_m[:nq], ours.q_v[:nq], "q", 0)
+        check(ref["q2"], opts["q_optimizer"], ours.q_params[nq:], ours.q_m[nq:], ours.q_v[nq:], "q", 0)
+        check(ref["q1_target"], None, ours.q_target_params[:nq], None, None, "q", 0)
+        check(ref["q2_target"], None, ours.q_target_params[nq:], None, None, "q", 0)
+
+    check_all(ref, opts)
+    assert torch.equal(ours.log_alpha.reshape(-1), ent.log_alpha.detach().reshape(-1))
+    st = opts["entropy_optimizer"].state[ent.log_alpha]
     assert float(ours.alpha_state[1]) == float(st["exp_avg"]) and float(ours.alpha_state[2]) == float(st["exp_avg_sq"]) and int(ours.steps[1]) == 3
-    nsd = ref.observation_normalizer.state_dict()
+    nsd = ref["observation_normalizer"].state_dict()
     assert torch.equal(ours.norm_mean.reshape(-1), nsd["running_mean"].reshape(-1)) and torch.equal(ours.norm_var.reshape(-1), nsd["running_var"].reshape(-1))
     assert int(ours.norm_count[0]) == int(nsd["count"])
 
-    # ---- and back: what the plugin writes, through the reference's own load()
+    # ---- and back: what the plugin writes, through the reference's load() sequence
     for t in (ours.policy_params, ours.q_params, ours.q_target_params, ours.policy_m, ours.q_m):
         t.add_(torch.randn(t.shape, generator=g) * 0.01)          # not the tensors that came in
     ours.save()
-    rcfg2 = ref_arm._ConfigDict(algorithm=ref_config("fastsac.pytorch"), environment=ref_arm._ConfigDict(seed=8, nr_envs=N),
-                                runner=ref_arm._ConfigDict(save_model=False, track_console=False, track_tb=False, track_wandb=False,
-                                                           load_model=os.path.join(str(tmp_path / "our_run"), "models", "latest.model")))
-    rcfg2.algorithm.device, rcfg2.algorithm.bf16_mixed_precision_training, rcfg2.algorithm.compile_mode = "cpu", False, "default"
-    back = reffs.FastSAC.load(rcfg2, Env(), Env(), str(tmp_path / "ref_run2"), None, ["algorithm.device", "algorithm.bf16_mixed_precision_training",
-                                                                                     "algorithm.compile_mode"])
-    ref = back
-    check(ref.policy, ref.policy_optimizer, ours.policy_params, ours.policy_m, ours.policy_v, "policy", 2)
-    check(ref.critic.q1, ref.q_optimizer, ours.q_params[:nq], ours.q_m[:nq], ours.q_v[:nq], "q", 0)
-    check(ref.critic.q2, ref.q_optimizer, ours.q_params[nq:], ours.q_m[nq:], ours.q_v[nq:], "q", 0)
-    check(ref.critic.q1_target, None, ours.q_target_params[:nq], None, None, "q", 0)
+    back, back_opts, back_ent = load_like_the_reference(os.path.join(str(tmp_path / "our_run"), "models", "latest.model"), layout)
+    check_all(back, back_opts)
+    assert torch.equal(ours.log_alpha.reshape(-1), back_ent.log_alpha.detach().reshape(-1))
+    bsd = back["observation_normalizer"].state_dict()
+    assert torch.equal(ours.norm_mean.reshape(-1), bsd["running_mean"].reshape(-1)) and int(ours.norm_count[0]) == int(bsd["count"])

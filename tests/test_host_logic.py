@@ -8,6 +8,8 @@ import numpy as np
 import pytest
 import torch
 
+from conftest import load_like_the_reference, reference_enums, reference_interfaces, reference_module, reference_optimizer
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -344,36 +346,30 @@ def test_checkpoint_written_by_the_reference_maps_onto_the_flat_layout():
 
 
 def test_checkpoint_written_here_loads_into_the_reference_modules():
-    """The other direction, with the reference's own classes (staged copy oracle/_ref): strict load_state_dict + optimizer.load_state_dict
-    as in the reference's load() (ppo.py:447-450)."""
-    from oracle import make_ref
-    if not make_ref.available():
-        pytest.skip("oracle/_ref not staged (python oracle/make_ref.py)")
-    from oracle import ref_arm
+    """The other direction: strict load_state_dict + optimizer.load_state_dict as in the reference's load() (ppo.py:447-450), into modules
+    and Adam optimizers laid out as the reference's (parameter names, shapes, order, optimizer numbering and settings captured from the
+    executed reference in tests/golden/reference_interfaces.json)."""
     from rl_x_b200 import _native as nt
-    from rl_x_b200.algorithms.ppo.b200.ppo import CRITIC_PARAM_ORDER, POLICY_PARAM_ORDER
-    os.environ["TORCHDYNAMO_DISABLE"] = "1"
-    refppo = ref_arm.import_reference()
-    from rl_x.algorithms.ppo.pytorch.default_config import get_config
-    ck, ex, k, fp = _ckpt_fixture()
-    N, T, obs, act, hid, mb, E = (int(x) for x in ex["meta"])
+    from rl_x_b200.algorithms.ppo.b200.kernels import PpoKernels
+    from rl_x_b200.algorithms.ppo.b200.ppo import CRITIC_PARAM_ORDER, FlatParameters, POLICY_PARAM_ORDER
+    ref = reference_interfaces()["checkpoints"]["ppo"]
+    meta = ref["meta"]
+    k = PpoKernels(meta["obs"], meta["act"], meta["hidden"])
+    fp = FlatParameters(k, "cpu")
     g = torch.Generator().manual_seed(0)
     fp.flat.copy_(torch.randn(k.param_count, generator=g))
     m1, m2 = torch.randn(k.param_count, generator=g), torch.rand(k.param_count, generator=g)
     pol, cri = fp.state_dicts()
-    a = get_config("ppo.pytorch")
-    a.device, a.bf16_mixed_precision_training, a.nr_steps, a.nr_epochs, a.minibatch_size, a.nr_hidden_units = "cpu", False, T, E, mb, hid
-    cfg = ref_arm._ConfigDict(algorithm=a, environment=ref_arm._ConfigDict(seed=0, nr_envs=N),
-                              runner=ref_arm._ConfigDict(save_model=False, track_console=False, track_tb=False, track_wandb=False))
-    env = ref_arm.SyntheticTorchEnv(N, obs, act)
-    model = refppo.PPO(cfg, env, env, "/tmp/rlx_ckpt_interop", None)
-    model.policy.load_state_dict(pol)
-    model.critic.load_state_dict(cri)
-    model.policy_optimizer.load_state_dict(fp.adam_state_dict(POLICY_PARAM_ORDER, nt.POLICY_KEYS, m1, m2, 5, 3e-4))
-    model.critic_optimizer.load_state_dict(fp.adam_state_dict(CRITIC_PARAM_ORDER, nt.CRITIC_KEYS, m1, m2, 5, 3e-4))
-    for net, opt, keys in ((model.policy, model.policy_optimizer, nt.POLICY_KEYS), (model.critic, model.critic_optimizer, nt.CRITIC_KEYS)):
+    policy, critic = reference_module(ref["modules"]["policy"]), reference_module(ref["modules"]["critic"])
+    policy.load_state_dict(pol)
+    critic.load_state_dict(cri)
+    popt = reference_optimizer(ref["optimizers"]["policy_optimizer"], {"": policy})
+    copt = reference_optimizer(ref["optimizers"]["critic_optimizer"], {"": critic})
+    popt.load_state_dict(fp.adam_state_dict(POLICY_PARAM_ORDER, nt.POLICY_KEYS, m1, m2, 5, 3e-4))
+    copt.load_state_dict(fp.adam_state_dict(CRITIC_PARAM_ORDER, nt.CRITIC_KEYS, m1, m2, 5, 3e-4))
+    for net, opt, keys in ((policy, popt, nt.POLICY_KEYS), (critic, copt, nt.CRITIC_KEYS)):
         for name, p in net.named_parameters():
-            seg = keys[name.replace("_orig_mod.", "")]
+            seg = keys[name]
             assert torch.equal(p.detach(), fp.view(fp.flat, seg)), name
             assert torch.equal(opt.state[p]["exp_avg"], fp.view(m1, seg)) and torch.equal(opt.state[p]["exp_avg_sq"], fp.view(m2, seg)), name
             assert float(opt.state[p]["step"]) == 5.0
@@ -566,110 +562,61 @@ def test_sac_checkpoint_written_by_the_reference_maps_onto_the_flat_layout():
         S._load_adam_state(bad, pol_views(m_p), pol_views(v_p), "policy")
 
 
-def test_sac_checkpoint_written_here_loads_into_the_reference_modules():
-    """The other direction for SAC, with the reference's own classes (staged copy oracle/_ref): the state dicts SAC.save() builds from the flat
-    buffers go through strict load_state_dict / optimizer.load_state_dict exactly as the reference's load() does (sac.py:398-416), and every
-    parameter / Adam moment ends up where its name says."""
-    from oracle import make_ref
-    if not make_ref.available():
-        pytest.skip("oracle/_ref not staged (python oracle/make_ref.py)")
-    from oracle import ref_arm
+def test_sac_checkpoint_written_here_loads_into_the_reference_modules(tmp_path):
+    """The other direction for SAC: the state dicts SAC.save() builds from the flat buffers go through strict load_state_dict /
+    optimizer.load_state_dict exactly as the reference's load() does (sac.py:398-416), into modules and optimizers laid out as the
+    reference's (tests/golden/reference_interfaces.json), and every parameter / Adam moment ends up where its name says."""
     from rl_x_b200.algorithms.sac.b200 import sac as S
-    os.environ["TORCHDYNAMO_DISABLE"] = "1"
-    ref_arm.import_reference()
-    import rl_x.algorithms.sac.pytorch.sac as refsac
-    from rl_x.algorithms.sac.pytorch.default_config import get_config
-    from rl_x.environments.action_space_type import ActionSpaceType
-    from rl_x.environments.data_interface_type import DataInterfaceType
-    from rl_x.environments.observation_space_type import ObservationSpaceType
-    N, obs, act, hid = 2, 5, 3, 16
-
-    class Props:
-        observation_space_type, action_space_type, data_interface_type = ObservationSpaceType.FLAT_VALUES, ActionSpaceType.CONTINUOUS, DataInterfaceType.NUMPY
-
-    class Env:
-        general_properties = Props
-        single_observation_space = ref_arm._Space((obs,))
-        single_action_space = ref_arm._Space((act,), np.full(act, -1.0, np.float32), np.full(act, 1.0, np.float32))
-
-    a = get_config("sac.pytorch")
-    a.device, a.bf16_mixed_precision_training, a.nr_hidden_units = "cpu", False, hid
-    cfg = ref_arm._ConfigDict(algorithm=a, environment=ref_arm._ConfigDict(seed=0, nr_envs=N),
-                              runner=ref_arm._ConfigDict(save_model=False, track_console=False, track_tb=False, track_wandb=False))
-    model = refsac.SAC(cfg, Env(), Env(), "/tmp/rlx_sac_ckpt_interop", None)
+    from rl_x_b200.algorithms.sac.b200.default_config import get_config
+    ref = reference_interfaces()["checkpoints"]["sac"]
+    obs, act, hid = ref["meta"]["obs"], ref["meta"]["act"], ref["meta"]["hidden"]
+    a = get_config("sac.b200")
+    a.nr_hidden_units = hid
     k = S.SacKernels(obs, act, hid, float(a.log_std_min), float(a.log_std_max))
     g = torch.Generator().manual_seed(1)
     policy, q = torch.randn(k.Pp, generator=g), torch.randn(4 * k.Pq, generator=g)
     m_p, v_p, m_q, v_q = torch.randn(k.Pp, generator=g), torch.rand(k.Pp, generator=g), torch.randn(4 * k.Pq, generator=g), torch.rand(4 * k.Pq, generator=g)
     pv, qv = k.policy_views(policy), k.q_views(q)
-    model.policy.load_state_dict({name: pv[name] for name in S.POLICY_PARAM_ORDER})
-    for net, mod in (("q1", model.critic.q1), ("q2", model.critic.q2), ("q1_target", model.critic.q1_target), ("q2_target", model.critic.q2_target)):
-        mod.load_state_dict(qv[net])
     pm, pvv = k.policy_views(m_p), k.policy_views(v_p)
     qm, qvv = k.q_views(m_q), k.q_views(v_q)
-    model.policy_optimizer.load_state_dict(S._adam_state_dict([pm[n] for n in S.POLICY_PARAM_ORDER], [pvv[n] for n in S.POLICY_PARAM_ORDER], 7, 3e-4))
-    model.q_optimizer.load_state_dict(S._adam_state_dict([qm[net][n] for net in ("q1", "q2") for n in S.Q_PARAM_ORDER],
-                                                         [qvv[net][n] for net in ("q1", "q2") for n in S.Q_PARAM_ORDER], 7, 3e-4))
-    model.entropy_optimizer.load_state_dict(S._adam_state_dict([torch.tensor([0.25])], [torch.tensor([0.5])], 7, 3e-4))
-    for name, p in model.policy.named_parameters():
-        name = name.replace("_orig_mod.", "")
-        st = model.policy_optimizer.state[p]
-        assert torch.equal(p.detach(), pv[name]) and torch.equal(st["exp_avg"], pm[name]) and torch.equal(st["exp_avg_sq"], pvv[name]), name
-        assert float(st["step"]) == 7.0
-    for net, mod in (("q1", model.critic.q1), ("q2", model.critic.q2)):
-        for name, p in mod.named_parameters():
-            name = name.replace("_orig_mod.", "")
-            st = model.q_optimizer.state[p]
-            assert torch.equal(p.detach(), qv[net][name]) and torch.equal(st["exp_avg"], qm[net][name]) and torch.equal(st["exp_avg_sq"], qvv[net][name]), (net, name)
-    st = model.entropy_optimizer.state[model.entropy_coefficient.log_alpha]
-    assert float(st["exp_avg"]) == 0.25 and float(st["exp_avg_sq"]) == 0.5 and float(st["step"]) == 7.0
-    # the whole file, as save() assembles it (checkpoint_dict), through the reference's own load() (sac.py:398-416): its assignment of
-    # checkpoint["log_alpha"] to a registered parameter only accepts an nn.Parameter
-    import tempfile
+    # the whole file, as save() assembles it (checkpoint_dict), through the reference's load(): its assignment of checkpoint["log_alpha"]
+    # to a registered parameter only accepts an nn.Parameter
     views = {"policy": ([pm[n] for n in S.POLICY_PARAM_ORDER], [pvv[n] for n in S.POLICY_PARAM_ORDER]),
              "q": ([qm[net][n] for net in ("q1", "q2") for n in S.Q_PARAM_ORDER], [qvv[net][n] for net in ("q1", "q2") for n in S.Q_PARAM_ORDER]),
              "entropy": ([torch.tensor([0.25])], [torch.tensor([0.5])])}
-    path = os.path.join(tempfile.mkdtemp(prefix="rlx_sac_ck_"), "best.model")
+    path = str(tmp_path / "best.model")
     torch.save(S.checkpoint_dict(a, {n: pv[n].clone() for n in pv}, {net: {n: t.clone() for n, t in d.items()} for net, d in qv.items()},
                                  torch.tensor([-0.7]), views, [7, 7, 7], 3e-4), path)
-    cfg.runner.load_model = path
-    back = refsac.SAC.load(cfg, Env(), Env(), "/tmp/rlx_sac_ckpt_interop2", None, ["algorithm.device", "algorithm.bf16_mixed_precision_training"])
-    assert isinstance(back.entropy_coefficient.log_alpha, torch.nn.Parameter) and float(back.entropy_coefficient.log_alpha.detach()) == pytest.approx(-0.7)
-    for name, p in back.policy.named_parameters():
-        assert torch.equal(p.detach(), pv[name.replace("_orig_mod.", "")]), name
-    for net, mod in (("q1", back.critic.q1), ("q2", back.critic.q2), ("q1_target", back.critic.q1_target), ("q2_target", back.critic.q2_target)):
-        for name, p in mod.named_parameters():
-            assert torch.equal(p.detach(), qv[net][name.replace("_orig_mod.", "")]), (net, name)
-    for name, p in back.critic.q2.named_parameters():
-        assert torch.equal(back.q_optimizer.state[p]["exp_avg_sq"], qvv["q2"][name.replace("_orig_mod.", "")]), name
+    mods, opts, ent = load_like_the_reference(path, ref)
+    assert isinstance(ent.log_alpha, torch.nn.Parameter) and float(ent.log_alpha.detach()) == pytest.approx(-0.7)
+    for name, p in mods["policy"].named_parameters():
+        st = opts["policy_optimizer"].state[p]
+        assert torch.equal(p.detach(), pv[name]) and torch.equal(st["exp_avg"], pm[name]) and torch.equal(st["exp_avg_sq"], pvv[name]), name
+        assert float(st["step"]) == 7.0
+    for net in ("q1", "q2", "q1_target", "q2_target"):
+        for name, p in mods[net].named_parameters():
+            assert torch.equal(p.detach(), qv[net][name]), (net, name)
+            if net in ("q1", "q2"):
+                st = opts["q_optimizer"].state[p]
+                assert torch.equal(st["exp_avg"], qm[net][name]) and torch.equal(st["exp_avg_sq"], qvv[net][name]), (net, name)
+    st = next(iter(opts["entropy_optimizer"].state.values()))
+    assert float(st["exp_avg"]) == 0.25 and float(st["exp_avg_sq"]) == 0.5 and float(st["step"]) == 7.0
 
 
 def test_plugins_pass_the_reference_runners_compatibility_check():
-    """Drop-in at the plugin level (INTEGRATION.md 1): this package's plugins registered into the REFERENCE's registry (staged copy of
-    rl_x/algorithms/algorithm_manager.py) and put through the expressions of the reference's runner (rl_x/runner/runner.py:86-101) with the
-    reference's own enum members on the environment side.  Those expressions use `in` / `==` on Enum members of two different packages,
-    which only holds because this package's enums equal same-named members of same-named foreign enums (environments/types.py: NamedEnum)."""
-    from oracle import make_ref
-    if not make_ref.available():
-        pytest.skip("oracle/_ref not staged (python oracle/make_ref.py)")
-    from oracle import ref_arm
-    ref_arm.import_reference()
-    from rl_x.algorithms import algorithm_manager as ref_manager
-    from rl_x.algorithms.deep_learning_framework_type import DeepLearningFrameworkType as RefFramework
-    from rl_x.environments.action_space_type import ActionSpaceType as RefAction
-    from rl_x.environments.data_interface_type import DataInterfaceType as RefInterface
-    from rl_x.environments.observation_space_type import ObservationSpaceType as RefObservation
-    from rl_x.environments.simulation_type import SimulationType as RefSimulation
+    """Drop-in at the plugin level (INTEGRATION.md 1): this package's plugins put through the expressions of the reference's runner
+    (rl_x/runner/runner.py:86-101) with the reference's enum members on the environment side.  Those expressions use `in` / `==` on Enum
+    members of two different packages, which only holds because this package's enums equal same-named members of same-named foreign enums
+    (environments/types.py: NamedEnum)."""
     import importlib
-    for algo, module, cls in (("ppo.b200", "ppo", "PPO"), ("espo.b200", "espo", "ESPO"), ("sac.b200", "sac", "SAC"), ("fastsac.b200", "fastsac", "FastSAC"),
-                              ("ppo_lstm.b200", "ppo_lstm", "PPO_LSTM")):
-        pkg = "rl_x_b200.algorithms." + algo
-        # the maintainer's four-line shim of INTEGRATION.md 1, with the reference's register_algorithm
-        ref_manager.register_algorithm(algo, importlib.import_module(pkg + ".default_config").get_config,
-                                       getattr(importlib.import_module(f"{pkg}.{module}"), cls),
-                                       importlib.import_module(pkg + ".general_properties").GeneralProperties)
-        props = ref_manager.get_algorithm_general_properties(algo)
-        assert ref_manager.get_algorithm_model_class(algo).__name__ == cls and ref_manager.get_algorithm_config(algo).name == algo
+    from rl_x_b200.algorithms.algorithm_manager import get_algorithm_config, get_algorithm_general_properties, get_algorithm_model_class
+    E = reference_enums()
+    RefAction, RefObservation, RefInterface = E["ActionSpaceType"], E["ObservationSpaceType"], E["DataInterfaceType"]
+    RefSimulation, RefFramework = E["SimulationType"], E["DeepLearningFrameworkType"]
+    for algo, cls in (("ppo.b200", "PPO"), ("espo.b200", "ESPO"), ("sac.b200", "SAC"), ("fastsac.b200", "FastSAC"), ("ppo_lstm.b200", "PPO_LSTM")):
+        importlib.import_module("rl_x_b200.algorithms." + algo)
+        props = get_algorithm_general_properties(algo)
+        assert get_algorithm_model_class(algo).__name__ == cls and get_algorithm_config(algo).name == algo
 
         class EnvProps:   # what a reference environment plugin states (e.g. custom_mujoco/ant/warp_torch/general_properties.py)
             action_space_type, observation_space_type = RefAction.CONTINUOUS, RefObservation.FLAT_VALUES
@@ -688,6 +635,12 @@ def test_plugins_pass_the_reference_runners_compatibility_check():
     from rl_x_b200.environments.synthetic.box.general_properties import GeneralProperties as BoxProps
     assert not (RefSimulation.JAX_BASED == BoxProps.simulation_type)
     assert BoxProps.action_space_type in [RefAction.CONTINUOUS, RefAction.DISCRETE] and BoxProps.data_interface_type in [RefInterface.NUMPY, RefInterface.TORCH]
+    # every member of the reference's enums exists here under the same name and value
+    from rl_x_b200.algorithms import deep_learning_framework_type as fw
+    from rl_x_b200.environments import types as env_types
+    for name, ref_enum in E.items():
+        ours = getattr(fw if name == "DeepLearningFrameworkType" else env_types, name)
+        assert {m.name: m.value for m in ours} == {m.name: m.value for m in ref_enum}, name
 
 
 def test_default_configs_are_ml_collections_config_dicts_where_available(monkeypatch):
@@ -722,67 +675,64 @@ def test_default_configs_are_ml_collections_config_dicts_where_available(monkeyp
     assert type(runner_config("train")) is FakeMlConfigDict
 
 
-def test_importing_a_plugin_package_registers_it_with_the_reference_too():
+def test_importing_a_plugin_package_registers_it_with_the_reference_too(tmp_path, monkeypatch):
     """No bridge package: the reference's runner does importlib.import_module(f"{package}.algorithms.{name}") for each implementation
-    package and then asks rl_x's OWN managers for the plugin (runner.py:232-247, 86-96).  With rl_x importable (here: the staged copy),
-    importing rl_x_b200's plugin packages must therefore leave them in rl_x's registries as well as in this package's."""
+    package and then asks rl_x's OWN managers for the plugin (runner.py:232-247, 86-96).  With rl_x importable (here: a stand-in whose
+    register functions take the reference's parameters, tests/golden/reference_interfaces.json), importing rl_x_b200's plugin packages must
+    therefore leave them in rl_x's registries as well as in this package's."""
     import importlib
-    from oracle import make_ref
-    if not make_ref.available():
-        pytest.skip("oracle/_ref not staged (python oracle/make_ref.py)")
-    from oracle import ref_arm
-    ref_arm.import_reference()
-    from rl_x.algorithms import algorithm_manager as ref_algorithms
-    from rl_x.environments import environment_manager as ref_environments
-    for name in ("ppo.b200", "espo.b200", "sac.b200", "fastsac.b200", "ppo_lstm.b200"):
-        ref_algorithms._algorithms.pop(name, None)
-        importlib.reload(importlib.import_module(f"rl_x_b200.algorithms.{name}"))       # what runner.import_algorithm does, from a clean slate
-        assert ref_algorithms.get_algorithm_model_class(name).__module__.startswith("rl_x_b200.algorithms." + name)
-        assert ref_algorithms.get_algorithm_config(name).name == name
-        assert ref_algorithms.get_algorithm_general_properties(name).deep_learning_framework_type.name == "TORCH"
-    for name in ("synthetic.box", "synthetic.pendulum"):
-        ref_environments._environments.pop(name, None)
-        importlib.reload(importlib.import_module(f"rl_x_b200.environments.{name}"))
-        assert callable(ref_environments.get_environment_create_train_and_eval_env(name))
-        assert ref_environments.get_environment_config(name).name == name
-        assert ref_environments.get_environment_general_properties(name).action_space_type.name == "CONTINUOUS"
+    registry = reference_interfaces()["registry"]
+    pkg = tmp_path / "rl_x"
+    for kind in ("algorithms", "environments"):
+        (pkg / kind).mkdir(parents=True)
+        (pkg / kind / "__init__.py").write_text("")
+        params = registry[f"register_{kind[:-1]}"]
+        (pkg / kind / f"{kind[:-1]}_manager.py").write_text(
+            f"_{kind} = {{}}\n\n\ndef register_{kind[:-1]}({', '.join(params)}):\n    _{kind}[name] = dict({', '.join(f'{p}={p}' for p in params)})\n")
+    (pkg / "__init__.py").write_text("")
+    monkeypatch.syspath_prepend(str(tmp_path))
+    is_rl_x = lambda m: m == "rl_x" or m.startswith("rl_x.")
+    for mod in [m for m in sys.modules if is_rl_x(m)]:
+        monkeypatch.delitem(sys.modules, mod)
+    try:
+        from rl_x.algorithms import algorithm_manager as ref_algorithms
+        from rl_x.environments import environment_manager as ref_environments
+        for name in ("ppo.b200", "espo.b200", "sac.b200", "fastsac.b200", "ppo_lstm.b200"):
+            importlib.reload(importlib.import_module(f"rl_x_b200.algorithms.{name}"))       # what runner.import_algorithm does
+            entry = ref_algorithms._algorithms[name]
+            assert entry["get_model_class"].__module__.startswith("rl_x_b200.algorithms." + name)
+            assert entry["get_default_config"](name).name == name
+            assert entry["general_properties"].deep_learning_framework_type.name == "TORCH"
+        for name in ("synthetic.box", "synthetic.pendulum"):
+            importlib.reload(importlib.import_module(f"rl_x_b200.environments.{name}"))
+            entry = ref_environments._environments[name]
+            assert callable(entry["create_train_and_eval_env"])
+            assert entry["get_default_config"](name).name == name
+            assert entry["general_properties"].action_space_type.name == "CONTINUOUS"
+    finally:
+        for mod in [m for m in sys.modules if is_rl_x(m)]:      # the stand-in leaves with this test
+            del sys.modules[mod]
 
 
 def test_default_configs_carry_every_reference_key_with_the_reference_value():
     """Every key of the reference's default_config.py of the five algorithms is present with the SAME default, except the one documented
     difference (bf16_mixed_precision_training: this build's default is the fp32 parity path); keys this build adds are not reference keys.
-    Reference modules: the staged copies (ppo, sac, fastsac) and, in the build container only, /root/reference for espo and ppo_lstm."""
+    The reference's defaults: tests/golden/reference_interfaces.json."""
     import importlib
-    import runpy
-    from oracle import make_ref, ref_arm
-    if not make_ref.available():
-        pytest.skip("oracle/_ref not staged (python oracle/make_ref.py)")
-    ref_arm._install_stub()
-    sources = {"ppo": os.path.join(make_ref.DST, "rl_x/algorithms/ppo/pytorch/default_config.py"),
-               "sac": os.path.join(make_ref.DST, "rl_x/algorithms/sac/pytorch/default_config.py"),
-               "fastsac": os.path.join(make_ref.DST, "rl_x/algorithms/fastsac/pytorch/default_config.py"),
-               "espo": "/root/reference/rl_x/algorithms/espo/pytorch/default_config.py",
-               "ppo_lstm": "/root/reference/rl_x/algorithms/ppo_lstm/flax/default_config.py"}
-    checked = 0
-    for algo, path in sources.items():
-        if not os.path.exists(path):
-            continue
-        ref = runpy.run_path(path)["get_config"]("x")
+    configs = reference_interfaces()["default_configs"]
+    assert sorted(configs) == ["espo", "fastsac", "ppo", "ppo_lstm", "sac"]
+    for algo, ref in configs.items():
         ours = importlib.import_module(f"rl_x_b200.algorithms.{algo}.b200.default_config").get_config("x")
         assert [k for k in ref if k not in ours] == [], algo
         different = {k: (ref[k], ours[k]) for k in ref if k != "name" and ref[k] != ours[k]}
         assert set(different) <= {"bf16_mixed_precision_training"}, (algo, different)
-        checked += 1
-    assert checked >= 3
 
 
 def test_model_classes_have_the_reference_classes_methods_and_signatures():
     """Duck typing is the boundary (SURVEY 8 b): every method of the reference's model class exists on this package's class with the same
-    parameter names (`load` may be a classmethod: the runner calls it on the class either way, runner.py:334-337).  Read from the sources."""
+    parameter names (`load` may be a classmethod: the runner calls it on the class either way, runner.py:334-337).  Read from the sources;
+    the reference's side is tests/golden/reference_interfaces.json."""
     import ast
-    from oracle import make_ref
-    if not make_ref.available():
-        pytest.skip("oracle/_ref not staged (python oracle/make_ref.py)")
 
     def methods(path, cls):
         for node in ast.walk(ast.parse(open(path).read())):
@@ -791,19 +741,13 @@ def test_model_classes_have_the_reference_classes_methods_and_signatures():
         raise AssertionError(f"no class {cls} in {path}")
 
     pkg = os.path.join(ROOT, "rl_x_b200", "algorithms")
-    cases = [("PPO", os.path.join(make_ref.DST, "rl_x/algorithms/ppo/pytorch/ppo.py"), [f"{pkg}/ppo/b200/ppo.py"]),
-             ("SAC", os.path.join(make_ref.DST, "rl_x/algorithms/sac/pytorch/sac.py"), [f"{pkg}/sac/b200/sac.py"]),
-             ("FastSAC", os.path.join(make_ref.DST, "rl_x/algorithms/fastsac/pytorch/fastsac.py"), [f"{pkg}/fastsac/b200/fastsac.py"]),
-             ("ESPO", "/root/reference/rl_x/algorithms/espo/pytorch/espo.py", [f"{pkg}/ppo/b200/ppo.py", f"{pkg}/espo/b200/espo.py"]),
-             ("PPO_LSTM", "/root/reference/rl_x/algorithms/ppo_lstm/flax/ppo_lstm.py", [f"{pkg}/ppo_lstm/b200/ppo_lstm.py"])]
-    checked = 0
-    for cls, ref_path, our_paths in cases:
-        if not os.path.exists(ref_path):
-            continue
-        ref, ours = methods(ref_path, cls), {}
+    reference = reference_interfaces()["methods"]
+    cases = [("PPO", [f"{pkg}/ppo/b200/ppo.py"]), ("SAC", [f"{pkg}/sac/b200/sac.py"]), ("FastSAC", [f"{pkg}/fastsac/b200/fastsac.py"]),
+             ("ESPO", [f"{pkg}/ppo/b200/ppo.py", f"{pkg}/espo/b200/espo.py"]), ("PPO_LSTM", [f"{pkg}/ppo_lstm/b200/ppo_lstm.py"])]
+    assert sorted(reference) == sorted(c for c, _ in cases)
+    for cls, our_paths in cases:
+        ref, ours = reference[cls], {}
         for p, c in zip(our_paths, ["PPO", cls] if len(our_paths) == 2 else [cls]):   # ESPO inherits PPO here
             ours.update(methods(p, c))
         assert [m for m in ref if m not in ours] == [], cls
         assert {m: (ref[m], ours[m]) for m in ref if ref[m] != ours[m]} == {}, cls
-        checked += 1
-    assert checked >= 3
