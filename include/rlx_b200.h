@@ -263,12 +263,6 @@ int rlx_comm_stage_f32(rlx_comm* c, const float* src, int64_t n, void* stream);
 /* out[i] = sum over ranks r = 0..world-1 (in that order) of rank r's send buffer [i], i < n <= nfloats.  Every rank must call
  * it the same number of times; the kernel spins on peer flags (and traps after ~20 s if a peer never arrives). */
 int rlx_comm_allreduce_sum_f32(rlx_comm* c, float* out, int64_t n, void* stream);
-/* 0 (default) and 1: one-shot kernel; 2: two-shot (2, 4 or 8 ranks) = reduce-scatter by peer loads (rank r sums chunk r of every send
- * slot) + all-gather by peer stores into every rank's result buffer: 2 (W-1)/W n floats per rank over NVLink instead of (W-1) n, at the
- * price of a second flag round.  Same summation order.  Experimental: slower than one-shot at the PPO gradient size even on 8 GPUs
- * (61 vs 49 us per exchange inside the epoch), verified bit-identical to one-shot at 2 ranks; on 8 ranks it passed the in-bench
- * sharded-vs-single parity check, but a rank failed tests/dist_check_comm.py's 2000-call stress loop (not diagnosed). */
-int rlx_comm_set_algorithm(rlx_comm* c, int algo);
 int rlx_comm_destroy(rlx_comm* c);
 
 /* Sharded form of rlx_ppo_update_epoch_f32: minibatch k covers this rank's counts[k] consecutive gathered rows and is divided by
@@ -278,10 +272,9 @@ int rlx_ppo_update_epoch_sharded_f32(const rlx_ppo_minibatch_args* first, int64_
                                      const int64_t* global_counts, rlx_comm* comm, void* stream);
 
 
-/* Loss head of rlx_ppo_minibatch_fwdbwd_f32: 0 = the fused SIMT kernel, 1 = the GEMM formulation of csrc/ppo_head_gemm.cu (logits and
- * dZ2 as GEMMs around one flat loss kernel; measured slower, kept as an opt-in), 2 = the fused kernel on the warp-level tensor path
+/* Loss head of rlx_ppo_minibatch_fwdbwd_f32: 0 (default) = the fused SIMT kernel, 2 = the fused kernel on the warp-level tensor path
  * (csrc/ppo_head_mma.cuh: both skinny products as 3xTF32 mma.sync tiles; fp32 mode, hidden 128/256/512, act <= 31 - other shapes and the
- * bf16 mode run engine 0).  Returns the engine in effect. */
+ * bf16 mode run engine 0).  Any other value is an error and leaves the setting unchanged.  Returns the engine in effect. */
 int rlx_set_head_engine(int engine);
 /* bf16-autocast mode of the PPO entry points (the reference's `bf16_mixed_precision_training`, ppo.py:98-107,123,155,208,253; its default).
  * on != 0: rlx_ppo_forward_f32 / rlx_critic_forward_f32 / rlx_ppo_minibatch_fwdbwd_f32 / rlx_gae_f32 round every value that torch's autocast
@@ -295,17 +288,6 @@ int rlx_set_autocast_bf16(int on);
  * update run on pairs (256 x 256 / 256 x 192 tiles); 2 (default, with fwd_bn = 128): the forward / dX GEMMs too, with fwd_bn-wide pair tiles
  * (128: double-buffered accumulators, 256: single; other values keep the current setting).  Returns the mode. */
 int rlx_set_tc_pair(int mode, int fwd_bn);
-/* 1: rlx_ppo_update_epoch_f32 runs gradient assembly + both grad norms + clip + Adam of a minibatch as ONE kernel (grid barrier in the
- * caller's workspace); 0 (default; measured faster on B200): the three separate kernels of rlx_ppo_minibatch_fwdbwd_f32 /
- * rlx_gradnorm_clip_adam_f32.  Returns the setting. */
-int rlx_set_fused_tail(int on);
-/* bring-up / test entry of the GEMM head on caller buffers: H2 [m, 2*hidden] (policy | critic halves), torch-layout head weights; outputs
- * dZ2 [m, 2*hidden], dhead [m, round_up(act+1, 4)] (dMean | dV | 0) and ONE partial block headpart [2*act + 5 + 2*hidden] =
- * db3p | db3c | dlogstd | pg vl kl cf sums | db2p | db2c.  scratch: >= m * (2*act + 8) + (m / 256 + 2) * max(2*hidden, 8) floats. */
-int rlx_debug_ppo_head_gemm_f32(int64_t m, int32_t hidden, int32_t act_dim, const float* H2, const float* W3p, const float* W3c, const float* b3p,
-                                const float* b3c, const float* logstd, const float* actions, const float* logp_old, const float* adv,
-                                const float* ret, const float* adv_stats, float inv_mg, float clip_range, float critic_coef,
-                                int32_t ratio_delta_metric, float* dZ2, float* dhead, float* headpart, float* scratch, void* stream);
 
 /* ------------------------------------------------------------------------------------------ PPO + LSTM path -- */
 /* SURVEY.md §8 a18: rl_x/algorithms/ppo_lstm/flax (policy.py:36-146, critic.py:18-30, ppo_lstm.py:107-231), including the two policy

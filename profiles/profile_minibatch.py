@@ -1,6 +1,6 @@
 """One PPO minibatch update (config-2 shapes) in isolation, for `ncu --set full` captures of every kernel on the update path.
 
-    ncu --set full --clock-control none --import-source on -k regex:rlx -s <11*warmup> -c 11 -o gpurun_out/prof python profiles/profile_minibatch.py [engine] [reps] [head: fused|gemm]
+    ncu --set full --clock-control none --import-source on -k regex:rlx -s <11*warmup> -c 11 -o minibatch_prof python profiles/profile_minibatch.py [engine] [reps]
 """
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -10,7 +10,6 @@ from rl_x_b200.algorithms.ppo.b200.kernels import PpoKernels, make_hparams
 engine = sys.argv[1] if len(sys.argv) > 1 else "tcgen05"
 reps = int(sys.argv[2]) if len(sys.argv) > 2 else 3
 nt.load().rlx_set_gemm_engine(1 if engine == "tcgen05" else 0)
-nt.load().rlx_set_head_engine(1 if (len(sys.argv) > 3 and sys.argv[3] == "gemm") else 0)
 obs, act, hidden, m = 376, 17, 256, 32768
 k = PpoKernels(obs, act, hidden)
 dev = "cuda"

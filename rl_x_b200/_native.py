@@ -166,8 +166,6 @@ _SIGNATURES = {
     "rlx_set_gae_tma": (C.c_int, [C.c_int]),
     "rlx_set_autocast_bf16": (C.c_int, [C.c_int]),
     "rlx_set_tc_pair": (C.c_int, [C.c_int, C.c_int]),
-    "rlx_set_fused_tail": (C.c_int, [C.c_int]),
-    "rlx_debug_ppo_head_gemm_f32": (C.c_int, [C.c_int64, C.c_int32, C.c_int32] + [C.c_void_p] * 11 + [C.c_float] * 3 + [C.c_int32] + [C.c_void_p] * 5),
     "rlx_get_gemm_engine": (C.c_int, []),
     "rlx_pcg64_seed": (C.c_int, [C.c_uint64, C.POINTER(Pcg64)]),
     "rlx_pcg64_next64": (C.c_uint64, [C.POINTER(Pcg64)]),
@@ -220,7 +218,6 @@ _SIGNATURES = {
     "rlx_comm_send_buffer": (C.c_void_p, [C.c_void_p]),
     "rlx_comm_stage_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "rlx_comm_allreduce_sum_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
-    "rlx_comm_set_algorithm": (C.c_int, [C.c_void_p, C.c_int]),
     "rlx_comm_destroy": (C.c_int, [C.c_void_p]),
     "rlx_ppo_update_epoch_sharded_f32": (C.c_int, [C.POINTER(PpoMinibatchArgs), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rlx_replay_sample_gather_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64] + [C.c_void_p] * 10 + [C.c_void_p]),

@@ -27,7 +27,7 @@ _DEFAULTS = (
     ('gemm_engine', "auto"),  # auto | simt (fp32 FFMA) | tcgen05 (3xTF32 tensor cores)
     ('exact_global_permutation', True),  # multi-GPU: reference-exact global shuffle (ppo.py:273-276) vs per-rank local shuffles
     ('gradient_exchange', "peer"),  # multi-GPU: peer (library all-reduce kernel over NVLink peer memory) | nccl (torch.distributed)
-    ('peer_exchange_algorithm', "auto"),  # auto = one_shot (measured fastest at 2 and 8 GPUs) | one_shot | two_shot (reduce-scatter / all-gather, experimental)
+    ('peer_exchange_algorithm', "auto"),  # auto | one_shot: both select the one-shot peer all-reduce kernel, the only one there is
     ('device_episode_statistics', True),  # TORCH-interface envs: episode return / length tracked on the device, read back once per iteration
     ('ignore_process_group', False),      # build a single-GPU instance inside a multi-rank job (bench.py's sharded-vs-single parity check)
     ('rollout_noise', "philox"),  # philox (in-kernel counter-based normals) | torch (torch.randn on device, injected)

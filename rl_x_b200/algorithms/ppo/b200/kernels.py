@@ -208,10 +208,6 @@ class PeerComm:
         n = out.numel() if n is None else int(n)
         nt.check(self.lib.rlx_comm_allreduce_sum_f32(self.handle, _f32(out, "out"), n, _stream()), "rlx_comm_allreduce_sum_f32")
 
-    def set_algorithm(self, algo):
-        """0 / 1: one-shot; 2: two-shot (experimental)."""
-        nt.check(self.lib.rlx_comm_set_algorithm(self.handle, int(algo)), "rlx_comm_set_algorithm")
-
     def close(self):
         if self.handle:
             self.lib.rlx_comm_destroy(self.handle)

@@ -228,6 +228,9 @@ class PPO:
         self.gradient_exchange = str(config.algorithm.get("gradient_exchange", "peer"))  # "peer": library kernel over NVLink; "nccl"
         if self.gradient_exchange not in ("peer", "nccl"):
             raise ValueError("gradient_exchange must be 'peer' or 'nccl'")
+        if str(config.algorithm.get("peer_exchange_algorithm", "auto")) not in ("auto", "one_shot"):
+            raise ValueError("peer_exchange_algorithm must be 'auto' or 'one_shot': the one-shot kernel is the only peer all-reduce "
+                             "(the two-shot kernel was removed)")
         self.peer_comm = None
         self._seg_cache = None
 
@@ -278,7 +281,6 @@ class PPO:
         if self.world_size > 1 and self.gradient_exchange == "peer" and self.peer_comm is None:
             try:
                 self.peer_comm = PeerComm(self.dist, P + nt.RLX_PPO_NMETRIC, self.device)
-                self.peer_comm.set_algorithm({"auto": 0, "one_shot": 1, "two_shot": 2}[str(config.algorithm.get("peer_exchange_algorithm", "auto"))])
             except RuntimeError as err:  # GPUs without peer access: NCCL carries the gradient instead (slower, same numbers up to sum order)
                 rlx_logger.warning(f"{err}; falling back to gradient_exchange='nccl'")
                 self.gradient_exchange = "nccl"

@@ -7,12 +7,10 @@ struct rlx_comm {
   int rank = 0, world = 1;
   int64_t nfloats = 0;
   size_t slot_bytes = 0;
-  uint8_t* base = nullptr;                       // own allocation: [flags 1 KiB][slot 0][slot 1][result]
+  uint8_t* base = nullptr;                       // own allocation: [flags 1 KiB][slot 0][slot 1]
   uint8_t* peer[RLX_COMM_MAX_WORLD] = {};        // mapped peer allocations (peer[rank] == base)
   uint64_t seq = 0;                              // all-reduces issued so far
   bool connected = false;
-  unsigned int* done = nullptr;                  // two-shot: per-device completion counter of the reduce-scatter phase (own memory)
-  int algo = 0;                                  // 0: pick by world size; 1: one-shot; 2: two-shot
 };
 
 namespace rlx {
@@ -24,7 +22,6 @@ constexpr int kThreads = 512;
 struct CommView {
   const float* slot[RLX_COMM_MAX_WORLD];          // every rank's send slot for this sequence number
   unsigned long long* flags[RLX_COMM_MAX_WORLD];  // every rank's flag array (flags[r][q]: rank q has published sequence number ...)
-  float* result[RLX_COMM_MAX_WORLD];              // two-shot: every rank's result buffer (this rank stores its reduced chunk into all of them)
 };
 // Optional side product of the all-reduce: per-net sums of squares of the REDUCED vector (the two clip_grad_norm_ norms of the PPO update),
 // one partial pair per CTA, so that no separate pass over the gradient is needed before clip + Adam.
@@ -131,100 +128,6 @@ __device__ __forceinline__ int comm_net_of(const CommSumsq& q, long long i) {
   for (int s = 1; s < RLX_PPO_NSEG; ++s) seg += (i >= q.seg_off[s]) ? 1 : 0;
   return (q.critic_mask >> seg) & 1u;
 }
-__device__ __forceinline__ void wait_flag(const unsigned long long* f, unsigned long long seq, int rank, int peer, const char* what) {
-  const unsigned long long t0 = global_ns();
-  while (ld_acquire_sys(f) < seq) {
-    if (global_ns() - t0 > 20000000000ull) {
-      printf("rlx_comm: rank %d waited 20 s for rank %d (%s) at sequence %llu\n", rank, peer, what, seq);
-      __trap();
-    }
-  }
-}
-
-// Two-shot all-reduce for larger worlds: (1) reduce-scatter - rank r sums chunk r of every rank's send slot straight from peer memory
-// (rank order => bit-identical everywhere) and STORES the reduced chunk into every rank's result buffer; (2) all-gather by those stores:
-// when every rank's chunk has landed, the full vector sits in local memory and is copied to `out` (with the optional sums of squares).
-// Per rank 2 (W-1)/W n floats cross NVLink instead of the one-shot kernel's (W-1) n.  Flags: flags[0..W) phase 1 (send slots ready),
-// flags[W..2W) phase 2 (chunks stored).  The result buffer needs no double buffering: a peer can only store chunk data of sequence s+1 after
-// this rank has published its send slot for s+1, which stream order puts after this kernel.
-template <int WORLD>
-__global__ void __launch_bounds__(kThreads) comm_allreduce2_kernel(CommView v, int rank, unsigned long long seq, float* __restrict__ out, long long n,
-                                                                    unsigned int* done, CommSumsq q) {
-  __shared__ float sh[34];
-  // ---- phase 1 barrier
-  if (blockIdx.x == 0 && threadIdx.x < WORLD) {
-    __threadfence_system();
-    st_release_sys(v.flags[threadIdx.x] + rank, seq);
-  }
-  if (threadIdx.x < WORLD) wait_flag(v.flags[rank] + threadIdx.x, seq, rank, (int)threadIdx.x, "send slot");
-  __syncthreads();
-  // ---- reduce-scatter: this rank's chunk, in float4 units (the tail chunk absorbs the remainder)
-  const long long n4 = n >> 2;
-  const long long per = (n4 + WORLD - 1) / WORLD;
-  const long long c0 = min(n4, per * rank), c1 = min(n4, c0 + per);
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = c0 + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < c1; i += stride) {
-    float4 x[WORLD];
-#pragma unroll
-    for (int r = 0; r < WORLD; ++r) x[r] = __ldcv(reinterpret_cast<const float4*>(v.slot[r]) + i);
-    float4 acc = x[0];
-#pragma unroll
-    for (int r = 1; r < WORLD; ++r) { acc.x += x[r].x; acc.y += x[r].y; acc.z += x[r].z; acc.w += x[r].w; }
-#pragma unroll
-    for (int r = 0; r < WORLD; ++r) reinterpret_cast<float4*>(v.result[r])[i] = acc;
-  }
-  if (rank == WORLD - 1 && blockIdx.x == 0) {  // scalar tail (n not a multiple of 4): the last rank owns it
-    for (long long i = (n4 << 2) + threadIdx.x; i < n; i += blockDim.x) {
-      float acc = __ldcv(v.slot[0] + i);
-      for (int r = 1; r < WORLD; ++r) acc += __ldcv(v.slot[r] + i);
-      for (int r = 0; r < WORLD; ++r) v.result[r][i] = acc;
-    }
-  }
-  // ---- phase 2 barrier: the LAST CTA of this rank to finish its stores publishes "chunk `rank` is in everybody's result buffer"
-  __threadfence_system();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int old = atomicAdd(done, 1u);
-    if (old == gridDim.x - 1) {
-      *done = 0u;
-      __threadfence_system();
-      for (int r = 0; r < WORLD; ++r) st_release_sys(v.flags[r] + WORLD + rank, seq);
-    }
-  }
-  if (threadIdx.x < WORLD) wait_flag(v.flags[rank] + WORLD + threadIdx.x, seq, rank, (int)threadIdx.x, "reduced chunk");
-  __syncthreads();
-  // ---- local copy result -> out, with the per-net sums of squares of the reduced gradient
-  const float* __restrict__ res = v.result[rank];
-  float sp = 0.f, sc = 0.f;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    const float4 a = __ldcv(reinterpret_cast<const float4*>(res) + i);
-    reinterpret_cast<float4*>(out)[i] = a;
-    if (q.partials != nullptr) {
-      const float e[4] = {a.x, a.y, a.z, a.w};
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const long long idx = 4 * i + j;
-        if (idx < q.total) { if (comm_net_of(q, idx)) sc = fmaf(e[j], e[j], sc); else sp = fmaf(e[j], e[j], sp); }
-      }
-    }
-  }
-  if (blockIdx.x == 0) {
-    for (long long i = (n4 << 2) + threadIdx.x; i < n; i += blockDim.x) {
-      const float a = __ldcv(res + i);
-      out[i] = a;
-      if (q.partials != nullptr && i < q.total) { if (comm_net_of(q, i)) sc = fmaf(a, a, sc); else sp = fmaf(a, a, sp); }
-    }
-  }
-  if (q.partials != nullptr) {
-    sp = block_sum(sp, sh);
-    sc = block_sum(sc, sh);
-    if (threadIdx.x == 0) {
-      q.partials[2 * blockIdx.x] = sp;
-      q.partials[2 * blockIdx.x + 1] = sc;
-      if (blockIdx.x == 0 && q.step_count != nullptr) q.step_count[0] += 1;
-    }
-  }
-}
 
 }  // namespace
 }  // namespace rlx
@@ -238,12 +141,10 @@ extern "C" int rlx_comm_create(int rank, int world, int64_t nfloats, rlx_comm** 
   rlx_comm* c = new rlx_comm();
   c->rank = rank; c->world = world; c->nfloats = nfloats;
   c->slot_bytes = align_up((size_t)nfloats * sizeof(float), 1024);
-  const size_t total = kFlagBytes + 3 * c->slot_bytes;  // flags | send slot 0 | send slot 1 | result buffer (two-shot)
-  static_assert(kFlagBytes >= 2 * RLX_COMM_MAX_WORLD * sizeof(unsigned long long), "flag area too small for two phases");
+  const size_t total = kFlagBytes + 2 * c->slot_bytes;  // flags | send slot 0 | send slot 1
+  static_assert(kFlagBytes >= RLX_COMM_MAX_WORLD * sizeof(unsigned long long), "flag area too small");
   cudaError_t e = cudaMalloc((void**)&c->base, total);  // plain cudaMalloc: exportable through cudaIpcGetMemHandle
   if (e == cudaSuccess) e = cudaMemset(c->base, 0, total);
-  if (e == cudaSuccess) e = cudaMalloc((void**)&c->done, 256);
-  if (e == cudaSuccess) e = cudaMemset(c->done, 0, 256);
   if (e == cudaSuccess) e = cudaDeviceSynchronize();
   if (e != cudaSuccess) {
     set_error("rlx_comm_create: CUDA error %s", cudaGetErrorString(e));
@@ -299,14 +200,8 @@ static int comm_allreduce(rlx_comm* c, float* out, int64_t n, void* stream, cons
 
 extern "C" int rlx_comm_allreduce_sum_f32(rlx_comm* c, float* out, int64_t n, void* stream) { return comm_allreduce(c, out, n, stream, nullptr, nullptr); }
 
-extern "C" int rlx_comm_set_algorithm(rlx_comm* c, int algo) {
-  RLX_CHECK_ARG(c != nullptr && algo >= 0 && algo <= 2, "bad arguments");
-  c->algo = algo;
-  return RLX_OK;
-}
-
-// PPO update: all-reduce of [gradient | metric sums] with the two squared gradient norms of the reduced gradient as a side product when the
-// two-shot kernel runs (returns the number of partial pairs written, 0 = none: the caller runs its own pass).
+// PPO update: all-reduce of [gradient | metric sums] with the two squared gradient norms of the reduced gradient as a side product at 2, 4
+// and 8 ranks (returns the number of partial pairs written, 0 = none: the caller runs its own pass).
 int comm_allreduce_ppo(rlx_comm* c, float* out, int64_t n, const rlx_ppo_dims& d, float* norm_partials, long long* step_count, void* stream,
                        int* nblk_out) {
   CommSumsq q{};
@@ -330,27 +225,6 @@ static int comm_allreduce(rlx_comm* c, float* out, int64_t n, void* stream, cons
   for (int r = 0; r < c->world; ++r) {
     v.slot[r] = (const float*)(c->peer[r] + kFlagBytes + (c->seq & 1) * c->slot_bytes);
     v.flags[r] = (unsigned long long*)c->peer[r];
-    v.result[r] = (float*)(c->peer[r] + kFlagBytes + 2 * c->slot_bytes);
-  }
-  // Two-shot only when asked for.  Measured inside the PPO epoch on 8 B200s (gpurun_out/r2_bench_8gpu*.json): 61 us per exchange against
-  // 49 us for the one-shot kernel - at 1.3 MB the second flag round costs more than the 8 MB of extra NVLink reads it saves.
-  const bool two_shot = c->algo == 2 && (c->world == 2 || c->world == 4 || c->world == 8);
-  if (two_shot) {
-    const int64_t n4c = std::max<int64_t>((n >> 2) / c->world, 1);
-    const unsigned grid2 = (unsigned)std::min<int64_t>(std::max<int64_t>(ceil_div(n4c, kThreads), 8), sm_count());
-    CommSumsq q{};
-    if (sumsq) q = *sumsq;
-#define RLX_COMM2_LAUNCH(W)                                                                                                          \
-  RLX_LAUNCH_C(KC_ALLREDUCE, 0, 4.0 * n * 3, comm_allreduce2_kernel<W>, grid2, kThreads, 0, stream, v, c->rank, (unsigned long long)c->seq, out, \
-               (long long)n, c->done, q)
-    switch (c->world) {
-      case 2: RLX_COMM2_LAUNCH(2); break;
-      case 4: RLX_COMM2_LAUNCH(4); break;
-      default: RLX_COMM2_LAUNCH(8); break;
-    }
-#undef RLX_COMM2_LAUNCH
-    if (nblk_out && sumsq && sumsq->partials) *nblk_out = (int)grid2;
-    return RLX_OK;
   }
   const int64_t n4 = std::max<int64_t>(n >> 2, 1);
   const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(n4, kThreads), sm_count());
@@ -377,7 +251,6 @@ extern "C" int rlx_comm_destroy(rlx_comm* c) {
   for (int r = 0; r < c->world; ++r)
     if (r != c->rank && c->peer[r]) cudaIpcCloseMemHandle(c->peer[r]);
   if (c->base) cudaFree(c->base);
-  if (c->done) cudaFree(c->done);
   delete c;
   return RLX_OK;
 }

@@ -11,7 +11,6 @@
 #include "gemm_simt.cuh"
 #include "gemm_dispatch.cuh"
 #include "ppo_head.cuh"
-#include "ppo_head_gemm.cuh"
 #include "ppo_head_mma.cuh"
 #include "ppo_optim.cuh"
 
@@ -109,8 +108,8 @@ static TrainPlan plan_train(const rlx_ppo_dims& d, long long m) {
   P.head_blocks = head_grid(m);
   P.head_npart = (int)(2 * A + 5 + 2 * H);
   P.wgrad_chunks = (int)ceil_div(m, kHeadWgradRows);
-  // one (policy, critic) partial pair per CTA of whichever kernel leaves the squared norms behind: the <= SM-count grids of the fused tail
-  // and of the exchange kernels, or the gradient-assembly grid (one CTA per 256 flat elements + one per 8 "tall" elements)
+  // one (policy, critic) partial pair per CTA of whichever kernel leaves the squared norms behind: the <= SM-count grid of the exchange
+  // kernel, the 64 CTAs of ppo_grad_sumsq_kernel, or the gradient-assembly grid (one CTA per 256 flat elements + one per 8 "tall" elements)
   P.norm_blocks = (int)std::max<long long>(std::max(64, sm_count()), ceil_div(make_layout(d).total(), 256) + ceil_div(2 * H + 2 * A + 1 + (A + 1) * H, 8) + 8);
   size_t o = 0;
   auto take = [&](size_t& off, size_t nfloats) {
@@ -198,12 +197,7 @@ static bool head_dims_ok(const rlx_ppo_dims& d) {
   return dims_ok(d) && d.hidden <= 1024 && head_smem_bytes(d, true) <= 200 * 1024;
 }
 
-int ppo_head_gemm_path(const HeadGemmArgs& a, cudaStream_t st);  // ppo_head_gemm.cu
-static int g_head_engine = 0;                                       // 0 fused SIMT kernel, 1 GEMM formulation, 2 fused mma.sync kernel (rlx_set_head_engine)
-// rlx_set_fused_tail(1): one-launch optimiser tail inside the epoch call.  Measured on B200 (round 2, gpurun_out/r2_bench3.json): SLOWER than the
-// three separate kernels (57 us vs 20 + 9 + 8 us per minibatch) - the <= SM-count grid that the grid barrier needs leaves too few threads
-// in flight for the split-K partial reads (25 MB per minibatch), which the 1287-CTA grad_reduce grid hides.  Kept as an opt-in.
-static int g_fused_tail = 0;
+static int g_head_engine = 0;  // 0 fused SIMT kernel, 2 fused mma.sync kernel (rlx_set_head_engine)
 
 static void fill_head_common(HeadP& h, const PpoLayout& L, const float* params, const float* H2, long long rows) {
   h.M = (int)rows; h.H = L.H; h.act = L.act;
@@ -317,14 +311,13 @@ static int launch_grad_reduce(const GradReduceP& r, cudaStream_t st) {
   return RLX_OK;
 }
 
-// `deferred`: when non-null the flat-gradient assembly is NOT launched; its parameters are returned for the fused optimiser tail.
 // `fuse_norms`: the assembly kernel also leaves the two squared clip norms in the workspace (off_barrier + 16 bytes) and bumps Adam's
 // step counter, so that clip + Adam can follow without the separate sum-of-squares launch.
-static int minibatch_fwdbwd(const rlx_ppo_minibatch_args* a, void* stream, GradReduceP* deferred, bool fuse_norms = false);
+static int minibatch_fwdbwd(const rlx_ppo_minibatch_args* a, void* stream, bool fuse_norms = false);
 
-extern "C" int rlx_ppo_minibatch_fwdbwd_f32(const rlx_ppo_minibatch_args* a, void* stream) { return minibatch_fwdbwd(a, stream, nullptr); }
+extern "C" int rlx_ppo_minibatch_fwdbwd_f32(const rlx_ppo_minibatch_args* a, void* stream) { return minibatch_fwdbwd(a, stream); }
 
-static int minibatch_fwdbwd(const rlx_ppo_minibatch_args* a, void* stream, GradReduceP* deferred, bool fuse_norms) {
+static int minibatch_fwdbwd(const rlx_ppo_minibatch_args* a, void* stream, bool fuse_norms) {
   int rc = check_mb_args(a, true);
   if (rc) return rc;
   const rlx_ppo_dims& d = a->dims;
@@ -386,26 +379,14 @@ static int minibatch_fwdbwd(const rlx_ppo_minibatch_args* a, void* stream, GradR
     const int dh_ld = (int)(ceil_div(A + 1, 4) * 4);
     const bool fast_head = (A <= 31) && (H % 2 == 0) && (H <= 1024);
     const double head_flops = 4.0 * m * H * (A + 1), head_bytes = 4.0 * m * (4.0 * H + 2.0 * A + 5);
-    // opt-in GEMM formulation of the head (ppo_head_gemm.cu); dZ1 is free until the dX GEMM and serves as its scratch
-    const bool gemm_head = fast_head && g_head_engine == 1 && !bf16 && head_gemm_scratch_floats(m, H, A) <= m * 2LL * H;
-    if (gemm_head) {
-      HeadGemmArgs ha{m, H, A, dh_ld, H2, a->params + L.off[W3P], a->params + L.off[W3C], a->params + L.off[B3P], a->params + L.off[B3C],
-                      a->params + L.off[LOGSTD], a->actions, a->log_probs, a->advantages, a->returns, a->adv_stats, inv_mg, a->hp.clip_range,
-                      a->hp.critic_coef, a->hp.ratio_delta_metric != 0.f ? 1 : 0, dZ2, dhead, headpart, dZ1};
-      rc = ppo_head_gemm_path(ha, st);
-      if (rc) return rc;
-      head_blocks = 1;  // the path writes ONE partial block in the fused kernel's layout
-    }
     if (fast_head) {
       HeadTrain2Extra ex{dh_ld};
       const bool vec_head = (H == 128 || H == 256 || H == 512);
       // fused head on the warp-level tensor path (ppo_head_mma.cuh): fp32 mode, <= 4 n-tiles of 8 head columns
       const int nt4 = (int)ceil_div(dh_ld, 8);
       const size_t smem4 = head4_smem_floats(H, A, nt4) * sizeof(float);
-      const bool mma_head = !gemm_head && vec_head && g_head_engine == 2 && !bf16 && nt4 <= 4 && smem4 <= 220 * 1024;
-      if (gemm_head) {
-        // loss, dZ2, dhead and the partial block are done
-      } else if (mma_head) {
+      const bool mma_head = vec_head && g_head_engine == 2 && !bf16 && nt4 <= 4 && smem4 <= 220 * 1024;
+      if (mma_head) {
         head_blocks = (int)std::min<long long>(ceil_div(m, 16 * kHead4RowTiles), (long long)P.head_blocks);
 #define RLX_HEAD4(H_, NT_)                                                                                                          \
   do {                                                                                                                              \
@@ -621,7 +602,7 @@ static int minibatch_fwdbwd(const rlx_ppo_minibatch_args* a, void* stream, GradR
   r.logstd = a->params + L.off[LOGSTD];
   r.metrics = a->metrics; r.m_local = (float)m;
   r.bf16 = bf16;
-  if (fuse_norms && deferred == nullptr) {
+  if (fuse_norms) {
     r.norm_partials = ws_ptr<float>(ws, P.off_norm);
     r.done = ws_ptr<unsigned int>(ws, P.off_barrier);
     r.norm_out = ws_ptr<float>(ws, P.off_barrier) + 4;
@@ -629,10 +610,6 @@ static int minibatch_fwdbwd(const rlx_ppo_minibatch_args* a, void* stream, GradR
     for (int i = 0; i <= RLX_PPO_NSEG; ++i) r.seg_off[i] = L.off[i];
     for (int i = 0; i < RLX_PPO_NSEG; ++i)
       if (seg_is_critic(i)) r.critic_mask |= (1u << i);
-  }
-  if (deferred != nullptr) {
-    *deferred = r;
-    return RLX_OK;
   }
   rc = launch_grad_reduce(r, st);
   if (rc) return rc;
@@ -678,28 +655,13 @@ extern "C" int rlx_ppo_update_epoch_f32(const rlx_ppo_minibatch_args* first, int
   const int64_t nmb = ceil_div(count, mb);
   const int A = first->dims.act_dim;
   const int64_t O = first->states_ld > 0 ? first->states_ld : first->dims.obs_dim;  // row pitch of the gathered states
-  // fused optimiser tail (ppo_optim.cuh): every thread of a <= SM-count grid keeps its gradient elements in registers across a grid
-  // barrier.  Needs the whole flat gradient to fit (kTailPerThread elements per thread) and the tall groups (head bias partials: 2H +
-  // 2A + 1 elements, W3 when it comes from the SIMT head) to fit two per warp; otherwise the three separate kernels run.
   cudaStream_t st = (cudaStream_t)stream;
-  bool fused = g_fused_tail && dims_ok(first->dims) && first->exp_avg && first->exp_avg_sq && first->lr && first->step_count && first->workspace;
-  const PpoLayout L = fused ? make_layout(first->dims) : PpoLayout{};
-  unsigned tail_grid = 0;
   // clip norms fused into the gradient-assembly kernel (needs the optimiser state and the ticket word in the workspace zeroed once)
-  bool norms_in_reduce = !fused && dims_ok(first->dims) && first->exp_avg && first->exp_avg_sq && first->lr && first->step_count && first->workspace;
+  bool norms_in_reduce = dims_ok(first->dims) && first->exp_avg && first->exp_avg_sq && first->lr && first->step_count && first->workspace;
   if (norms_in_reduce) {
     const TrainPlan P0 = plan_train(first->dims, std::max<int64_t>(std::min<int64_t>(mb, count), 1));
     if (first->workspace_bytes < P0.total) norms_in_reduce = false;
     else RLX_CHECK_CUDA(cudaMemsetAsync(ws_ptr<unsigned int>(first->workspace, P0.off_barrier), 0, 64, st));
-  }
-  if (fused) {
-    tail_grid = (unsigned)std::min<int64_t>(sm_count(), ceil_div(L.total(), kTailThreads));
-    fused = (int64_t)tail_grid * kTailThreads * kTailPerThread >= L.total();
-    if (fused) {
-      const TrainPlan P0 = plan_train(first->dims, std::max<int64_t>(std::min<int64_t>(mb, count), 1));
-      if (first->workspace_bytes < P0.total) fused = false;  // the per-minibatch checks below will report it
-      else RLX_CHECK_CUDA(cudaMemsetAsync(ws_ptr<unsigned int>(first->workspace, P0.off_barrier), 0, 64, st));
-    }
   }
   for (int64_t k = 0; k < nmb; ++k) {
     rlx_ppo_minibatch_args a = *first;
@@ -713,9 +675,9 @@ extern "C" int rlx_ppo_update_epoch_f32(const rlx_ppo_minibatch_args* first, int
     a.returns = first->returns + r0;
     a.adv_stats = first->adv_stats + 2 * k;
     a.metrics = first->metrics ? first->metrics + RLX_PPO_NMETRIC * k : nullptr;
-    if (!fused && norms_in_reduce && a.m == std::min<int64_t>(mb, count)) {
-      // default: the assembly kernel leaves the clip norms behind; clip + Adam read them (no separate sum-of-squares launch)
-      int rc = minibatch_fwdbwd(&a, stream, nullptr, true);
+    if (norms_in_reduce && a.m == std::min<int64_t>(mb, count)) {
+      // the assembly kernel leaves the clip norms behind; clip + Adam read them (no separate sum-of-squares launch)
+      int rc = minibatch_fwdbwd(&a, stream, true);
       if (rc) return rc;
       const PpoLayout La = make_layout(a.dims);
       const TrainPlan Pa = plan_train(a.dims, std::max<int64_t>(a.m, 1));
@@ -725,28 +687,11 @@ extern "C" int rlx_ppo_update_epoch_f32(const rlx_ppo_minibatch_args* first, int
       RLX_LAUNCH_C(KC_CLIP_ADAM, 0, 28.0 * La.total(), ppo_clip_adam_kernel, (unsigned)ceil_div(La.total(), 256), 256, 0, st, ap);
       continue;
     }
-    if (!fused || a.m != std::min<int64_t>(mb, count)) {  // a short last minibatch has its own workspace plan: separate kernels
-      int rc = rlx_ppo_minibatch_fwdbwd_f32(&a, stream);
-      if (rc) return rc;
-      rc = rlx_gradnorm_clip_adam_f32(&a, stream);
-      if (rc) return rc;
-      continue;
-    }
-    TailP t{};
-    int rc = minibatch_fwdbwd(&a, stream, &t.r);
+    // a short last minibatch (it has its own workspace plan) or no optimiser state: separate kernels
+    int rc = rlx_ppo_minibatch_fwdbwd_f32(&a, stream);
     if (rc) return rc;
-    if (tall_elements(t.r) > 2LL * tail_grid * (kTailThreads / 32)) {  // more per-CTA partial columns than two per warp: separate kernels
-      rc = launch_grad_reduce(t.r, st);
-      if (rc) return rc;
-      rc = rlx_gradnorm_clip_adam_f32(&a, stream);
-      if (rc) return rc;
-      continue;
-    }
-    const TrainPlan P = plan_train(a.dims, std::max<int64_t>(a.m, 1));
-    t.a = make_adam_params(&a, L, P);
-    t.a.nblk_norm = (int)tail_grid;
-    t.barrier = ws_ptr<unsigned int>(a.workspace, P.off_barrier);
-    RLX_LAUNCH_C(KC_CLIP_ADAM, 0, partial_bytes(t.r) + 28.0 * L.total(), ppo_fused_tail_kernel, tail_grid, kTailThreads, 0, st, t);
+    rc = rlx_gradnorm_clip_adam_f32(&a, stream);
+    if (rc) return rc;
   }
   return RLX_OK;
 }
@@ -776,7 +721,7 @@ extern "C" int rlx_ppo_update_epoch_sharded_f32(const rlx_ppo_minibatch_args* fi
     a.metrics = send + P;
     int rc = rlx_ppo_minibatch_fwdbwd_f32(&a, stream);
     if (rc) return rc;
-    // the two-shot exchange kernel leaves the per-net squared norms of the reduced gradient behind (and bumps Adam's step counter):
+    // the exchange kernel leaves the per-net squared norms of the reduced gradient behind (and bumps Adam's step counter):
     // clip + Adam follow directly, without a separate pass over the gradient
     const TrainPlan TP = plan_train(a.dims, std::max<int64_t>(a.m, 1));
     int nblk = 0;
@@ -832,14 +777,9 @@ extern "C" int rlx_debug_gemm_f32(int engine, int layout, int epilogue, int64_t 
 }
 
 extern "C" int rlx_set_head_engine(int engine) {
-  if (engine >= 0 && engine <= 2) g_head_engine = engine;
+  if (engine == 0 || engine == 2) g_head_engine = engine;
   else set_error("rlx_set_head_engine: unknown engine %d", engine);
   return g_head_engine;
-}
-
-extern "C" int rlx_set_fused_tail(int on) {
-  g_fused_tail = on ? 1 : 0;
-  return g_fused_tail;
 }
 
 extern "C" int rlx_set_gemm_engine(int engine) {

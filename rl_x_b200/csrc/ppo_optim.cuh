@@ -277,179 +277,4 @@ __global__ void __launch_bounds__(1024) median_lower_kernel(const float* __restr
   if (threadIdx.x == 0) out[0] = s_nan ? __int_as_float(0x7FC00000) : __uint_as_float(s_prefix);
 }
 
-// ------------------------------------------------------------------------------------------------ fused optimiser tail
-// grad_reduce + grad_sumsq + clip_adam of one minibatch in ONE launch (they were three: 20 + 9 + 8 us, each dominated by launch and
-// DRAM round-trip latency on 1.3 MB of data).  Every thread keeps the <= kTailPerThread gradient elements it assembled in registers
-// across a grid-wide barrier, so the flat gradient is written once (for the caller / the logs) and never re-read.
-//   phase 1  assemble the gradient elements (same fixed summation orders as ppo_grad_reduce_kernel => same bits), per-net sum of squares
-//   barrier  block partials -> global, arrive on a counter; the last block bumps a generation word, everybody else spins on it.  All
-//            blocks are co-resident (grid <= SM count, 1 block fits per SM), and kernels behind this one in the stream cannot start
-//            before it ends, so the spin cannot deadlock.
-//   phase 2  every block sums the block partials in index order (=> identical norms everywhere), clip coefficients, Adam
-constexpr int kTailThreads = 512;
-constexpr int kTailPerThread = 8;
-
-struct TailP {
-  GradReduceP r;
-  AdamP a;
-  unsigned int* barrier;  // [2]: arrival counter, generation; zeroed by the caller before the first launch of an epoch
-};
-
-__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-__global__ void __launch_bounds__(kTailThreads) ppo_fused_tail_kernel(const TailP p) {
-  __shared__ float sh[34];
-  __shared__ float s_coef[2];
-  __shared__ float s_sc[2];
-  const GradReduceP& r = p.r;
-  const AdamP& a = p.a;
-  const int lane = threadIdx.x & 31;
-  const long long nthreads = (long long)gridDim.x * blockDim.x;
-  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const unsigned int gen0 = (threadIdx.x == 0) ? ld_acquire_u32(p.barrier + 1) : 0u;
-  // Adam's step counter is read by every block BEFORE the barrier (the previous minibatch's store is ordered by the stream) and stored by
-  // block 0 AFTER it: no block can still be waiting to read the old value then.
-  if (threadIdx.x == 32) {
-    // torch/optim/adam.py (_single_tensor_adam): step_size = lr / (1 - beta1^t); denom = sqrt(v)/sqrt(1 - beta2^t) + eps
-    const double t = (double)(a.step_count[0] + 1);
-    s_sc[0] = (float)((double)a.lr[0] / (1.0 - pow((double)a.beta1, t)));
-    s_sc[1] = (float)sqrt(1.0 - pow((double)a.beta2, t));
-  }
-
-  // ---- phase 1a: flat elements (few partials per element), one element per thread per pass
-  float g[kTailPerThread];
-  bool mine[kTailPerThread];
-  float sp = 0.f, sc = 0.f;
-#pragma unroll
-  for (int k = 0; k < kTailPerThread; ++k) {
-    const long long i = tid + (long long)k * nthreads;
-    g[k] = 0.f;
-    mine[k] = false;
-    if (i < r.total) {
-      bool own = true;
-      float s = 0.f;
-#pragma unroll
-      for (int gi = 0; gi < kNumGroups; ++gi) {
-        const GradGroup& gg = r.g[gi];
-        if (i >= gg.off && i < gg.off + gg.len) {
-          if (gg.nsplit > kTallSplit) own = false;
-          else s = grad_sum_serial(gg.src + (i - gg.off), gg.nsplit, gg.stride);
-        }
-      }
-      if (own) {
-        if (i >= r.logstd_off && i < r.logstd_off + r.act) s += r.entropy_grad;
-        else s = bf16r_if(s, r.bf16);
-        g[k] = s;
-        mine[k] = true;
-        r.grads[i] = s;
-        if (adam_net_of(a, i)) sc = fmaf(s, s, sc); else sp = fmaf(s, s, sp);
-      }
-    }
-  }
-  // ---- phase 1b: tall groups (hundreds of per-CTA partials per element): one warp per element, result lives in lane 0
-  float tg[2] = {0.f, 0.f};
-  long long ti[2] = {-1, -1};
-  const long long nwarps = nthreads >> 5;
-#pragma unroll
-  for (int k = 0; k < 2; ++k) {
-    long long w = (tid >> 5) + (long long)k * nwarps;
-#pragma unroll
-    for (int gi = 0; gi < kNumGroups; ++gi) {
-      const GradGroup& gg = r.g[gi];
-      if (gg.nsplit <= kTallSplit) continue;
-      if (w >= 0 && w < gg.len) {
-        float s = grad_sum_warp(gg.src + w, gg.nsplit, gg.stride, lane);
-        const long long i = gg.off + w;
-        if (i >= r.logstd_off && i < r.logstd_off + r.act) s += r.entropy_grad;
-        else s = bf16r_if(s, r.bf16);
-        if (lane == 0) {
-          tg[k] = s;
-          ti[k] = i;
-          r.grads[i] = s;
-          if (adam_net_of(a, i)) sc = fmaf(s, s, sc); else sp = fmaf(s, s, sp);
-        }
-        w = -1;
-      } else if (w >= gg.len) {
-        w -= gg.len;
-      }
-    }
-  }
-  // ---- metric sums of this minibatch (as ppo_grad_reduce_kernel's block 0)
-  if (blockIdx.x == 0 && r.metrics != nullptr) {
-    const int npart = r.npart, wi = threadIdx.x >> 5;
-    if (wi < 4) {
-      float s = 0.f;
-      for (int b = lane; b < r.nblk; b += 32) s += r.head_partials[(long long)b * npart + 2 * r.act + 1 + wi];
-      s = warp_sum(s) * r.inv_mg;
-      if (lane == 0) {
-        if (wi == 0) r.metrics[0] = s;
-        if (wi == 1) r.metrics[1] = r.critic_coef * s;
-        if (wi == 2) r.metrics[3] = s;
-        if (wi == 3) r.metrics[4] = s;
-      }
-    }
-    if (threadIdx.x == 128) {
-      float e = 0.f;
-      for (int q = 0; q < r.act; ++q) e += 0.5f + 0.5f * 1.8378770664093453f + logf(expf(r.logstd[q]));
-      r.metrics[2] = e * (r.m_local * r.inv_mg);
-      r.metrics[7] = r.m_local;
-    }
-  }
-  // ---- block partials of the two squared norms, then the grid barrier
-  sp = block_sum(sp, sh);
-  sc = block_sum(sc, sh);
-  if (threadIdx.x == 0) {
-    a.norm_partials[2 * blockIdx.x] = sp;
-    a.norm_partials[2 * blockIdx.x + 1] = sc;
-    __threadfence();
-    const unsigned int old = atomicAdd(p.barrier, 1u);
-    if (old == gridDim.x - 1) {
-      p.barrier[0] = 0u;  // ready for the next launch
-      __threadfence();
-      atomicAdd(p.barrier + 1, 1u);
-    } else {
-      while (ld_acquire_u32(p.barrier + 1) == gen0) {}
-    }
-    __threadfence();
-  }
-  __syncthreads();
-  // ---- phase 2: norms (fixed order), clip coefficients, bias corrections, Adam on the elements held in registers
-  if (blockIdx.x == 0 && threadIdx.x == 64) a.step_count[0] += 1;
-  if (threadIdx.x < 64) {
-    // warp 0: policy, warp 1: critic.  Lanes stride over the block partials (all loads in flight), then the fixed shuffle tree:
-    // the same order in every block => identical clip coefficients everywhere.
-    const int net = threadIdx.x >> 5;
-    float s = 0.f;
-    for (unsigned int b = lane; b < gridDim.x; b += 32) s += __ldcg(a.norm_partials + 2 * b + net);
-    s = warp_sum(s);
-    if (lane == 0) {
-      const float norm = sqrtf(s);
-      // clip_grad_norm_: clip_coef = max_norm / (total_norm + 1e-6), clamped to 1  (torch/nn/utils/clip_grad.py)
-      s_coef[net] = fminf(a.max_norm / (norm + 1e-6f), 1.f);
-      if (blockIdx.x == 0 && a.metrics != nullptr) a.metrics[5 + net] = norm;
-    }
-  }
-  __syncthreads();
-  auto adam = [&](long long i, float grad) {
-    const float gq = grad * s_coef[adam_net_of(a, i)];
-    float m = a.m[i], v = a.v[i];
-    m = m + (gq - m) * (1.f - a.beta1);
-    v = v * a.beta2 + (1.f - a.beta2) * gq * gq;
-    const float denom = sqrtf(v) / s_sc[1] + a.eps;
-    a.params[i] = a.params[i] - s_sc[0] * (m / denom);
-    a.m[i] = m;
-    a.v[i] = v;
-  };
-#pragma unroll
-  for (int k = 0; k < kTailPerThread; ++k)
-    if (mine[k]) adam(tid + (long long)k * nthreads, g[k]);
-#pragma unroll
-  for (int k = 0; k < 2; ++k)
-    if (ti[k] >= 0) adam(ti[k], tg[k]);
-}
-
 }  // namespace rlx

@@ -21,7 +21,6 @@ sys.path.insert(0, ROOT)
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--time", action="store_true")
-    ap.add_argument("--two-shot", action="store_true", help="also run the two-shot kernel at world sizes other than 2")
     ap.add_argument("--n", type=int, default=329_259)  # the Humanoid PPO gradient + 8 metric sums: not a multiple of 4
     args = ap.parse_args()
     from rl_x_b200.algorithms.ppo.b200.kernels import PeerComm
@@ -34,52 +33,35 @@ def main():
     comm = PeerComm(dist, n, dev)
     out = torch.empty(n, device=dev)
     idx = torch.arange(n, device=dev, dtype=torch.float32) % 97.0
-    # the two-shot kernel is an opt-in experiment (slower at this size, see include/rlx_b200.h): stress it where it is known to hold (2 ranks)
-    # or when asked for explicitly
-    algos = [(1, "one-shot")] + ([(2, "two-shot")] if (world == 2 or args.two_shot) and world in (2, 4, 8) else [])
-    results = {}
-    for algo, algo_name in algos:
-        comm.set_algorithm(algo)
-        # 1. exact sums, many calls in flight (also alternating with the other algorithm's slots / flags from the previous round)
-        calls = 2000
-        bad = torch.zeros(1, device=dev)
-        rank_sum = world * (world - 1) / 2.0
-        for c in range(calls):
-            src = idx * float(rank + 1) + float((c % 13) * (rank + 2))
-            comm.stage(src)
-            comm.allreduce_sum(out)
-            expect = idx * float(rank_sum + world) + float((c % 13) * (rank_sum + 2 * world))
-            bad += (out != expect).sum()
-        assert int(bad.item()) == 0, f"rank {rank} ({algo_name}): {int(bad.item())} wrong elements over {calls} calls"
-
-        # 2. random inputs: against NCCL, and identical bits everywhere
-        g = torch.Generator(device=dev).manual_seed(100 + rank)
-        src = torch.randn(n, device=dev, generator=g)
+    # 1. exact sums, many calls in flight
+    calls = 2000
+    bad = torch.zeros(1, device=dev)
+    rank_sum = world * (world - 1) / 2.0
+    for c in range(calls):
+        src = idx * float(rank + 1) + float((c % 13) * (rank + 2))
         comm.stage(src)
         comm.allreduce_sum(out)
-        ref = src.clone()
-        dist.all_reduce(ref)
-        rel = float((out - ref).norm() / ref.norm())
-        assert rel < 1e-6, rel
-        gathered = [torch.empty_like(out) for _ in range(world)]
-        dist.all_gather(gathered, out)
-        for r in range(world):
-            assert torch.equal(gathered[r], gathered[0]), f"rank {r} differs from rank 0 ({algo_name})"
-        results[algo] = out.clone()
-    if len(results) == 2:
-        assert torch.equal(results[1], results[2]), "one-shot and two-shot all-reduce disagree (both sum in rank order)"
+        expect = idx * float(rank_sum + world) + float((c % 13) * (rank_sum + 2 * world))
+        bad += (out != expect).sum()
+    assert int(bad.item()) == 0, f"rank {rank}: {int(bad.item())} wrong elements over {calls} calls"
+
+    # 2. random inputs: against NCCL, and identical bits everywhere
+    g = torch.Generator(device=dev).manual_seed(100 + rank)
+    src = torch.randn(n, device=dev, generator=g)
+    comm.stage(src)
+    comm.allreduce_sum(out)
+    ref = src.clone()
+    dist.all_reduce(ref)
+    rel = float((out - ref).norm() / ref.norm())
+    assert rel < 1e-6, rel
+    gathered = [torch.empty_like(out) for _ in range(world)]
+    dist.all_gather(gathered, out)
+    for r in range(world):
+        assert torch.equal(gathered[r], gathered[0]), f"rank {r} differs from rank 0"
 
     if args.time:
-        from rl_x_b200 import _native as nt
-        def peer(algo):
-            def run():
-                comm.allreduce_sum(out)
-            run.algo = algo
-            return run
-        timed = [(f"peer {nm}", peer(a)) for a, nm in algos] + [("nccl", lambda: dist.all_reduce(ref))]
+        timed = [("peer", lambda: comm.allreduce_sum(out)), ("nccl", lambda: dist.all_reduce(ref))]
         for name, fn in timed:
-            if hasattr(fn, "algo"):
-                comm.set_algorithm(fn.algo)
             for _ in range(50):
                 fn()
             dist.barrier()

@@ -78,9 +78,7 @@ def run_model(world, rank, local, engine, exchange="peer", single=False):
     dev = torch.device("cuda", local)
     a = get_config("ppo.b200")
     a.nr_steps, a.minibatch_size, a.nr_epochs, a.nr_hidden_units, a.total_timesteps = T, MB, EPOCHS, HID, NG * T * ITERS
-    # "peer2": the peer exchange with the two-shot kernel forced (its default use starts at 4 ranks), incl. the fused squared norms
-    a.entropy_coef, a.gemm_engine, a.gradient_exchange = 0.01, engine, ("peer" if exchange == "peer2" else exchange)
-    a.peer_exchange_algorithm = "two_shot" if exchange == "peer2" else "auto"
+    a.entropy_coef, a.gemm_engine, a.gradient_exchange = 0.01, engine, exchange
     a.ignore_process_group = bool(single)
     cfg = ConfigDict(algorithm=a, environment=ConfigDict(seed=5, nr_envs=nl),
                      runner=ConfigDict(save_model=False, track_console=False, track_tb=False, track_wandb=False, load_model=""))
@@ -100,9 +98,8 @@ def run_model(world, rank, local, engine, exchange="peer", single=False):
     model.rank = 0 if single else model.rank  # a `single` instance logs whatever its rank in the job is
     model.train()
     if world > 1:
-        want = "peer" if exchange == "peer2" else exchange
-        assert model.gradient_exchange == want, f"asked for the {want} exchange, ran {model.gradient_exchange}"
-        assert (model.peer_comm is not None) == (want == "peer")
+        assert model.gradient_exchange == exchange, f"asked for the {exchange} exchange, ran {model.gradient_exchange}"
+        assert (model.peer_comm is not None) == (exchange == "peer")
     pol, cri = model.params.state_dicts()
     if world > 1:  # peers may still be reading this rank's exchange slots: nobody frees them before everybody is done
         torch.cuda.synchronize()
@@ -159,7 +156,7 @@ if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--out")
     ap.add_argument("--engine", default="auto")
-    ap.add_argument("--exchange", default="peer", choices=["peer", "peer2", "nccl"])
+    ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"])
     ap.add_argument("--compare", nargs=2)
     args = ap.parse_args()
     if args.compare:

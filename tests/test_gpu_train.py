@@ -321,7 +321,7 @@ def test_load_checkpoint_written_by_the_reference(tmp_path, monkeypatch):
     assert list(ck["policy_state_dict"])[0] == "policy_logstd" and tuple(ck["policy_optimizer_state_dict"]["state"][0]["exp_avg"].shape) == (1, act)
 
 
-@pytest.mark.parametrize("exchange", ["peer", "peer2", "nccl"])
+@pytest.mark.parametrize("exchange", ["peer", "nccl"])
 def test_two_gpu_sharded_run_equals_single_gpu_run(tmp_path, gemm_engine, exchange):
     """Env-sharded data parallelism over 2 GPUs reproduces the 1-GPU run on the same global batch, with the gradient carried by
     the library's peer-memory all-reduce kernel ("peer") or by NCCL ("nccl")."""

@@ -1,53 +1,11 @@
-"""Opt-in GEMM formulation of the PPO loss head (rlx_set_head_engine(1), csrc/ppo_head_gemm.cu) inside rlx_ppo_minibatch_fwdbwd_f32:
-gradients and metrics must equal the default fused-kernel head's.  Host emulation of the same source: tests/test_lstm_emulation.py::test_emulated_ppo_head_gemm_path.
-First passed on a B200 at the round-1 driver run; strict since round 2."""
+"""Opt-in mma.sync formulation of the PPO loss head (rlx_set_head_engine(2), csrc/ppo_head_mma.cuh) inside rlx_ppo_minibatch_fwdbwd_f32:
+gradients and metrics must equal the default fused SIMT head's."""
 import numpy as np
 import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
-
-
-@pytest.mark.parametrize("obs,act,hidden,m", [(376, 17, 256, 4096), (24, 5, 128, 1000)])
-def test_gemm_head_matches_fused_head(obs, act, hidden, m):
-    from rl_x_b200 import _native as nt
-    from rl_x_b200.algorithms.ppo.b200.kernels import PpoKernels, make_hparams
-    from oracle import ppo_oracle as O
-    from rl_x_b200.algorithms.ppo.b200.ppo import FlatParameters
-    lib = nt.load()
-    k = PpoKernels(obs, act, hidden)
-    pol, cri = O.init_params(obs, act, hidden, seed=3)
-    fp = FlatParameters(k, DEV)
-    fp.load_named({**pol, **cri})
-    g = torch.Generator().manual_seed(1)
-    ldx = k.states_pitch()
-    states = torch.zeros(m, ldx)
-    states[:, :obs] = torch.randn(m, obs, generator=g)
-    states[:, obs] = 1.0
-    t = lambda x: x.to(DEV).contiguous()
-    actions, logp, adv, ret = t(torch.randn(m, act, generator=g)), t(torch.randn(m, generator=g) * 0.3 - act), t(torch.randn(m, generator=g)), t(torch.randn(m, generator=g))
-    stats = torch.tensor([float(adv.mean()), float(adv.std())], device=DEV)
-    P = k.param_count
-    results = []
-    try:
-        for engine in (0, 1):
-            assert lib.rlx_set_head_engine(engine) == engine
-            grads, metrics = torch.zeros(P, device=DEV), torch.zeros(nt.RLX_PPO_NMETRIC, device=DEV)
-            args = k.minibatch_args(m=m, m_global=m, states=t(states), actions=actions, log_probs=logp, advantages=adv, returns=ret, adv_stats=stats,
-                                    params=fp.flat, grads=grads, exp_avg=torch.zeros(P, device=DEV), exp_avg_sq=torch.zeros(P, device=DEV),
-                                    lr=torch.full((1,), 3e-4, device=DEV), step_count=torch.zeros(1, dtype=torch.int64, device=DEV),
-                                    hp=make_hparams(0.2, 0.01, 0.5, 0.5), metrics=metrics, workspace=k.minibatch_workspace(m, DEV), states_ld=ldx,
-                                    states_ones_col=True)
-            k.fwdbwd(args)
-            torch.cuda.synchronize()
-            results.append((grads.cpu().numpy(), metrics.cpu().numpy()))
-    finally:
-        lib.rlx_set_head_engine(0)
-    (g0, m0), (g1, m1) = results
-    rel = float(np.linalg.norm(g1 - g0) / np.linalg.norm(g0))
-    assert rel <= 2e-5, rel
-    np.testing.assert_allclose(m1[:5], m0[:5], rtol=2e-4, atol=2e-6)
 
 
 def _run_head_engine(lib, k, fp, engine, m, ldx, states, actions, logp, adv, ret, stats, hp):

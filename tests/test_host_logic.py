@@ -161,6 +161,17 @@ def test_ppo_refuses_to_run_without_cuda():
         PPO(r._config, train_env, eval_env, "/tmp/x", None)
 
 
+def test_ppo_rejects_unknown_peer_exchange_algorithm():
+    """algorithm.peer_exchange_algorithm accepts auto | one_shot (the one-shot kernel is the only peer all-reduce); anything else is
+    refused before anything runs."""
+    from rl_x_b200.runner.runner import Runner
+    from rl_x_b200.algorithms.ppo.b200.ppo import PPO
+    r = Runner(argv=["--environment.nr_envs=8", "--algorithm.nr_steps=4", "--algorithm.minibatch_size=8", "--algorithm.peer_exchange_algorithm=ring"])
+    train_env, eval_env = r._create_train_and_eval_env(r._config)
+    with pytest.raises(ValueError, match="peer_exchange_algorithm must be 'auto' or 'one_shot'"):
+        PPO(r._config, train_env, eval_env, "/tmp/x", None)
+
+
 @pytest.mark.parametrize("algo", ["sac.b200", "fastsac.b200", "ppo_lstm.b200"])
 def test_non_identity_observation_indices_are_rejected_not_ignored(algo):
     """SURVEY §8 a20: the reference index-selects the network inputs with env.policy_observation_indices / critic_observation_indices

@@ -512,61 +512,6 @@ def test_emulated_nstep_replay_matches_reference_golden(tmp_path):
                 assert np.array_equal(got, ref), f"{tag}/{name} vs reference"
 
 
-@pytest.mark.parametrize("m,hid,act,rd", [(300, 16, 3, 0), (1000, 64, 17, 0), (257, 32, 6, 1)])
-def test_emulated_ppo_head_gemm_path(tmp_path, m, hid, act, rd):
-    """rl_x_b200/csrc/ppo_head_gemm.cu (the opt-in GEMM formulation of the PPO loss head) compiled for the host, against autograd of the PPO
-    loss (ppo.py:121-160) from the layer-2 activations: dZ2, the dW3 operand dhead, and the partial block (bias / log-std gradients,
-    metric sums) in the layout the rest of the update consumes."""
-    out = tmp_path / "libheadgemm_emu.so"
-    subprocess.run(emu_build_cmd(out, os.path.join(ROOT, "rl_x_b200", "csrc", "ppo_head_gemm.cu")), check=True)
-    lib = C.CDLL(str(out))
-    lib.rlx_debug_ppo_head_gemm_f32.argtypes = ([C.c_int64, C.c_int32, C.c_int32] + [C.c_void_p] * 11 + [C.c_float] * 3 + [C.c_int32] +
-                                                [C.c_void_p] * 5)
-    torch.manual_seed(m)
-    clip, cc = 0.2, 0.5
-    Z2 = (torch.randn(m, 2 * hid) * 0.8).requires_grad_(True)
-    W3p, W3c = (torch.randn(act, hid) * 0.3).requires_grad_(True), (torch.randn(1, hid) * 0.3).requires_grad_(True)
-    b3p, b3c = (torch.randn(act) * 0.1).requires_grad_(True), (torch.randn(1) * 0.1).requires_grad_(True)
-    logstd = (torch.randn(act) * 0.2).requires_grad_(True)
-    actions, logp_old = torch.randn(m, act), torch.randn(m) * 0.3 - act
-    adv, ret = torch.randn(m), torch.randn(m)
-    stats = torch.tensor([float(adv.mean()), float(adv.std())])
-    H2 = torch.tanh(Z2)
-    mean = H2[:, :hid] @ W3p.t() + b3p
-    value = (H2[:, hid:] @ W3c.t() + b3c).reshape(-1)
-    std = torch.exp(logstd)
-    logp = (-((actions - mean) ** 2) / (2 * std ** 2) - logstd - 0.5 * np.log(2 * np.pi)).sum(1)
-    logratio = logp - logp_old
-    ratio = logratio.exp()
-    An = (adv - stats[0]) / (stats[1] + 1e-8)
-    pg = torch.maximum(-An * ratio, -An * torch.clamp(ratio, 1 - clip, 1 + clip))
-    vl = 0.5 * (value - ret) ** 2
-    loss = pg.mean() + cc * vl.mean()   # the entropy term has no H2 dependence; the update adds its log-std gradient separately
-    mean.retain_grad()
-    value.retain_grad()
-    loss.backward()
-    f = lambda t: np.ascontiguousarray(t.detach().numpy(), dtype=np.float32)
-    dh_ld = (act + 1 + 3) // 4 * 4
-    dZ2, dhead, part = np.zeros((m, 2 * hid), np.float32), np.full((m, dh_ld), np.nan, np.float32), np.zeros(2 * act + 5 + 2 * hid, np.float32)
-    scratch = np.zeros(m * (2 * act + 8) + (m // 256 + 2) * max(2 * hid, 8) + 64, np.float32)
-    ins = [f(H2), f(W3p), f(W3c), f(b3p), f(b3c), f(logstd), f(actions), f(logp_old), f(adv), f(ret), f(stats)]
-    rc = lib.rlx_debug_ppo_head_gemm_f32(m, hid, act, *[x.ctypes.data for x in ins], 1.0 / m, clip, cc, rd, dZ2.ctypes.data, dhead.ctypes.data,
-                                         part.ctypes.data, scratch.ctypes.data, None)
-    assert rc == 0
-    tol = dict(rtol=2e-4, atol=2e-7)
-    np.testing.assert_allclose(dZ2, f(Z2.grad), **tol)
-    np.testing.assert_allclose(dhead[:, :act], f(mean.grad), **tol)
-    np.testing.assert_allclose(dhead[:, act], f(value.grad), **tol)
-    assert np.all(dhead[:, act + 1:] == 0)
-    np.testing.assert_allclose(part[:act], f(b3p.grad), rtol=2e-4, atol=2e-6)
-    np.testing.assert_allclose(part[act], f(b3c.grad)[0], rtol=2e-4, atol=2e-6)
-    np.testing.assert_allclose(part[act + 1:2 * act + 1], f(logstd.grad), rtol=2e-4, atol=2e-6)
-    cf = (torch.abs(ratio - 1)).sum() if rd else (torch.abs(ratio - 1) > clip).float().sum()
-    sums = [float(t.detach()) for t in (pg.sum(), vl.sum(), ((ratio - 1) - logratio).sum(), cf)]
-    np.testing.assert_allclose(part[2 * act + 1:2 * act + 5], sums, rtol=2e-4, atol=1e-4)
-    np.testing.assert_allclose(part[2 * act + 5:], f(Z2.grad).sum(0), rtol=2e-4, atol=2e-6)
-
-
 def test_persistent_recurrence_is_race_free_under_tsan(tmp_path):
     """The one-launch-per-direction recurrence kernels (lstm_seq_fwd_kernel / lstm_seq_bwd_kernel: shared memory + one barrier per step) under
     ThreadSanitizer: the emulation runs each CUDA thread of a block as an OS thread and __syncthreads as a real barrier, so a barrier missing
